@@ -9,6 +9,10 @@ reference's only prover entry point (/root/reference/src/test_utils.rs:37-51).  
 
   python bench.py [--gpus N] [--steps K] [--warmup W]       # this repo's CUDA path
   python bench.py --impl reference [...]                     # CPU restatement (oracle/), per-phase sampled, same workload
+  python bench.py --dump-outputs DIR [...]                   # also write the last timed proof as DIR/proof.npy
+
+The prover's RNG is keyed by a fixed seed, so with the same arguments every run proves the same witness with the same
+blinding and the last timed proof is the same bytes: two builds can be compared output for output.
 
 N > 1 (torchrun, one rank per GPU) is STRONG scaling of the same single proof: sharded_backend.ShardedGpuBackend divides the
 commitments, the Lagrange -> coefficient transforms, the lookups, the permutation chunks and the quotient (NTTs by column
@@ -37,6 +41,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 K_LOG = int(os.environ.get("TRP_BENCH_K", "20"))          # 20 is the benchmark; smaller values are for dry runs of this file
 WORD_BITS = 32 if K_LOG >= 17 else 2 * (K_LOG - 2)
@@ -49,10 +54,11 @@ WORKLOAD = (f"one plonk.create_proof of the reference's TinyRamCircuit<{WORD_BIT
 FMUL_PER_MIXED_ADD = 10          # XYZZ madd-2008-s: 8M + 2S (SURVEY.md 8d)
 MACS_PER_FMUL = 128              # generic 8x8-limb CIOS: 64 product + 64 reduction 32x32->64 MACs
 DTYPE = "u32x8 (255-bit Montgomery)"
+RNG_SEED = hashlib.sha256(b"bench.py create_proof").digest()
 
 
 def _config(extra=None):
-    c = {"workload": WORKLOAD, "k": K_LOG, "word_bits": WORD_BITS, "curve": "vesta", "rng": "AES-256-CTR keyed by an OS seed (rank 0's, broadcast); random polynomials = a 32-byte key of that stream expanded on the device (BLAKE2b counter mode)",
+    c = {"workload": WORKLOAD, "k": K_LOG, "word_bits": WORD_BITS, "curve": "vesta", "rng": "AES-256-CTR keyed by a fixed seed (RNG_SEED); random polynomials = a 32-byte key of that stream expanded on the device (BLAKE2b counter mode)",
          "l2_policy": "inputs larger than L2 (15.5 GiB of per-proof polynomials at k = 20)"}
     if extra:
         c.update(extra)
@@ -340,7 +346,7 @@ def run_gpu(args):
     t0 = time.perf_counter()
     pk = PL.keygen(be, cs, d_fixed, copies)
     be._wait(); t_keygen = time.perf_counter() - t0
-    rng = ShardedRng(be.p, d, "cuda")                                      # rank 0's OS seed, the same stream on every rank
+    rng = ShardedRng(be.p, d, "cuda", seed=RNG_SEED)                       # the same stream on every rank and in every run
 
     def barrier():
         if world > 1:
@@ -385,6 +391,8 @@ def run_gpu(args):
     elapsed_ms = float(t.item())
     seconds = elapsed_ms * 1e-3 / args.steps
     value = 1.0 / seconds
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, proof)
 
     # ---- end to end: the witness starts in pinned host memory every step, the proof bytes end on the host ----------------------------
     up = torch.empty_like(block)
@@ -503,6 +511,12 @@ def run_gpu(args):
         dist.destroy_process_group()
     ok = verified and same
     sys.exit(0 if ok else 1)
+
+
+def dump_outputs(out_dir, proof: bytes):
+    """What a caller of create_proof receives from the last timed step: the serialized proof, one float32 per byte (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "proof.npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float32))
 
 
 def measure_extras(pkg, ctx, stream, peaks, peak_src, int_peak_tmacs):
@@ -628,8 +642,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the MSM and NTT lines that follow the headline (N = 1)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the sampled CPU baseline (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step as DIR/proof.npy (float32, one per byte)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs: the reference arm samples phase timings and produces no proof")
         run_reference(args)
     else:
         run_gpu(args)
