@@ -171,6 +171,9 @@ int trp_quotient_eval(trp_domain* d, const uint32_t* program, size_t n_instr, un
 /* out[i] = p(zeta * extended_omega^(j + i * 2^(extended_k-k))) for coefficient-form columns p (n each): row j, j + 2^(..),
  * ... of coeff_to_extended, computed with ONE size-n NTT per column. */
 int trp_dev_coeff_to_coset(trp_domain* d, const uint64_t* d_coeff, uint64_t* d_out, size_t batch, unsigned coset);
+/* The same for columns anywhere in device memory: d_src_tab is a DEVICE array of batch column addresses, column i's values go
+ * to d_out[i * n ..] (which must not overlap a source).  Expands a subset of a prover's columns with no staging copy. */
+int trp_dev_coeff_to_coset_gather(trp_domain* d, const uint64_t* const* d_src_tab, uint64_t* d_out, size_t batch, unsigned coset);
 /* OR into trp_dev_quotient_eval's coset index: write the coset's n results contiguously at d_out[row] instead of
  * interleaving them into the extended vector (input layout of trp_dev_cosets_to_coeff). */
 #define TRP_Q_CONTIGUOUS 0x10000
@@ -179,6 +182,12 @@ int trp_dev_coeff_to_coset(trp_domain* d, const uint64_t* d_coeff, uint64_t* d_o
  * extended_to_coeff(divide_by_vanishing_poly(h_ext)) while only ncos = j - 1 of the 2^(extended_k - k) cosets are ever
  * evaluated: the quotient h(X) is unique, so commitments and proof bytes are unchanged. */
 int trp_dev_cosets_to_coeff(trp_domain* d, uint64_t* d_vals, unsigned ncos, uint64_t* d_out_coeff, int divide_by_vanishing);
+/* The same for h = sum_p h_p given part by part, deg h_p < n * ncos[p] <= n * ncos_out: part p brings its values on the first
+ * ncos[p] cosets (d_vals: the parts' rows back to back, sum_p ncos[p] x n; consumed), the ncos_out x n coefficients of h are
+ * written to d_out_coeff.  A quotient numerator split by constraint degree is evaluated only on the cosets each part needs;
+ * h is unique, so the result equals trp_dev_cosets_to_coeff of the whole numerator on ncos_out cosets.  1 <= n_parts <= 64. */
+int trp_dev_cosets_to_coeff_parts(trp_domain* d, uint64_t* d_vals, const unsigned* ncos /* host, n_parts */, unsigned n_parts,
+                                  unsigned ncos_out, uint64_t* d_out_coeff, int divide_by_vanishing);
 
 /* ---- between the hot kernels (SURVEY.md 8(f) row f1): the grand products and the lookup permutation of create_proof -------
  * halo2_proofs 0.2.0 plonk/permutation/prover.rs (Argument::commit), plonk/lookup/prover.rs (Argument::commit_permuted,

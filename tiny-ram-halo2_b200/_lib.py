@@ -26,7 +26,8 @@ EXPORTED_SYMBOLS = [
     "trp_domain_create", "trp_domain_free", "trp_domain_extended_k", "trp_domain_constants",
     "trp_lagrange_to_coeff", "trp_dev_lagrange_to_coeff", "trp_coeff_to_lagrange",
     "trp_coeff_to_extended", "trp_dev_coeff_to_extended", "trp_extended_to_coeff", "trp_dev_extended_to_coeff",
-    "trp_dev_quotient_eval", "trp_dev_quotient_eval_rows", "trp_quotient_eval", "trp_dev_coeff_to_coset", "trp_dev_cosets_to_coeff",
+    "trp_dev_quotient_eval", "trp_dev_quotient_eval_rows", "trp_quotient_eval", "trp_dev_coeff_to_coset", "trp_dev_coeff_to_coset_gather",
+    "trp_dev_cosets_to_coeff", "trp_dev_cosets_to_coeff_parts",
     "trp_field_op", "trp_dev_field_op", "trp_microbench",
     "trp_dev_batch_invert", "trp_batch_invert", "trp_dev_grand_product", "trp_grand_product",
     "trp_dev_permutation_product", "trp_permutation_product", "trp_dev_lookup_product", "trp_lookup_product",
@@ -111,7 +112,9 @@ def load_library():
     L.trp_dev_quotient_eval_rows.argtypes = [vp, vp, sz, u, vp, sz, vp, sz, u, sz, sz, u, u, vp]
     L.trp_quotient_eval.argtypes = [vp, vp, sz, u, vp, sz, vp, sz, vp]
     L.trp_dev_coeff_to_coset.argtypes = [vp, vp, vp, sz, u]
+    L.trp_dev_coeff_to_coset_gather.argtypes = [vp, vp, vp, sz, u]
     L.trp_dev_cosets_to_coeff.argtypes = [vp, vp, u, vp, i]
+    L.trp_dev_cosets_to_coeff_parts.argtypes = [vp, vp, vp, u, u, vp, i]
     L.trp_field_op.argtypes = [vp, i, i, vp, vp, vp, sz]
     L.trp_dev_field_op.argtypes = [vp, i, i, vp, vp, vp, sz]
     L.trp_microbench.argtypes = [vp, i, i, ctypes.POINTER(ctypes.c_double)]

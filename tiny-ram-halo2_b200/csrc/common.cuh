@@ -45,10 +45,15 @@ struct trp_ctx {
   void* pinned = nullptr;
   size_t pinned_bytes = 0;
   std::vector<TwiddleTable> twiddles;
-  // quotient.cu: the caller's last quotient program and its lowered form (qlower.h); a prover runs one program on j - 1 cosets
-  std::vector<uint32_t> q_src, q_low, q_staged;
-  unsigned q_src_regs = 0, q_low_regs = 0;
-  size_t q_src_consts = 0;
+  // quotient.cu: the caller's last few quotient programs and their lowered forms (qlower.h), most recent first; a prover runs
+  // one program per constraint degree on each coset it needs, the same programs proof after proof
+  struct QProgram {
+    std::vector<uint32_t> src, low;
+    unsigned src_regs = 0, low_regs = 0;
+    size_t src_consts = 0;
+  };
+  std::vector<QProgram> q_progs;
+  std::vector<uint32_t> q_staged;
 };
 
 struct trp_bases {
@@ -161,7 +166,8 @@ inline size_t ws_align(size_t b) { return (b + 255) & ~(size_t)255; }
 int trp_ntt_impl(trp_ctx* ctx, int field, const void* d_src, void* d_dst, size_t batch, unsigned log_n,
                  const uint64_t omega[4], size_t src_stride, size_t dst_stride, unsigned n_src,
                  const void* d_pre, unsigned pre_period, const void* d_post, unsigned post_period, unsigned n_dst,
-                 void* d_tmp /* batch*2^log_n elements, needed iff src==dst and passes>1 */);
+                 void* d_tmp /* batch*2^log_n elements, needed iff src==dst and passes>1 */,
+                 const void* const* d_src_tab = nullptr /* DEVICE table of batch column addresses read instead of d_src */);
 size_t trp_ntt_passes(unsigned log_n);
 int trp_get_powers(trp_ctx* ctx, int field, unsigned log_n, const uint64_t g[4], const void** out);
 int trp_msm_impl(trp_ctx* ctx, const trp_bases* bases, const void* d_scalars, size_t n, size_t m, void* d_out_jac,

@@ -38,6 +38,7 @@ struct NttPass {
   unsigned n_src, n_dst;
   const uint4* pre; unsigned pre_period;
   const uint4* post; unsigned post_period;
+  const uint4* const* src_tab;     // first pass only, or NULL: column y of the batch is read from src_tab[y] (src unused)
 };
 
 template <class PR>
@@ -62,7 +63,7 @@ __global__ void __launch_bounds__(NTT_THREADS) ntt_pass_kernel(NttPass p) {
   uint4* plane0 = smem;
   uint4* plane1 = smem + nelem;
   const unsigned g = blockIdx.x;
-  const uint4* src = p.src + 2 * (size_t)blockIdx.y * p.src_stride;
+  const uint4* src = p.src_tab ? p.src_tab[blockIdx.y] : p.src + 2 * (size_t)blockIdx.y * p.src_stride;
   uint4* dst = p.dst + 2 * (size_t)blockIdx.y * p.dst_stride;
   const unsigned smask = (1u << s) - 1, cmask = (1u << c) - 1;
 
@@ -150,7 +151,7 @@ __global__ void __launch_bounds__(NTT_THREADS, R >= 3 ? 2 : 3) ntt_pass_reg_kern
   uint4* plane0 = smem;
   uint4* plane1 = smem + nelem;
   const unsigned g = blockIdx.x;
-  const uint4* src = p.src + 2 * (size_t)blockIdx.y * p.src_stride;
+  const uint4* src = p.src_tab ? p.src_tab[blockIdx.y] : p.src + 2 * (size_t)blockIdx.y * p.src_stride;
   uint4* dst = p.dst + 2 * (size_t)blockIdx.y * p.dst_stride;
   const unsigned cmask = (1u << c) - 1;
   unsigned low_base = 0, hi = 0;
@@ -469,7 +470,7 @@ int get_twiddles(trp_ctx* ctx, unsigned log_n, const uint64_t omega[4], const ui
 template <class PR>
 int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned L, const uint64_t omega[4],
             size_t src_stride, size_t dst_stride, unsigned n_src, const void* d_pre, unsigned pre_period,
-            const void* d_post, unsigned post_period, unsigned n_dst, void* d_tmp) {
+            const void* d_post, unsigned post_period, unsigned n_dst, void* d_tmp, const void* const* d_src_tab) {
   if (batch == 0) return TRP_OK;
   if (L > 30) TRP_FAIL(ctx, TRP_E_INVALID, "log_n = %u is out of range (max 30)", L);
   if (batch > 65535) TRP_FAIL(ctx, TRP_E_INVALID, "batch = %zu exceeds 65535 columns per call", batch);
@@ -498,6 +499,7 @@ int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned
     size_t in_stride = p.first ? src_stride : mid_stride;
     size_t out_stride = p.last ? dst_stride : mid_stride;
     p.src = (const uint4*)in; p.dst = (uint4*)out; p.src_stride = in_stride; p.dst_stride = out_stride;
+    p.src_tab = p.first ? (const uint4* const*)d_src_tab : nullptr;
     unsigned nelem = 1u << (p.s + p.c);
     unsigned threads = nelem / 2 < NTT_THREADS ? nelem / 2 : NTT_THREADS;
     if (threads < 32) threads = 32;
@@ -519,7 +521,7 @@ int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned
       static const bool use_tma = [] { const char* e = getenv("TRP_NTT_TMA"); return e && atoi(e) == 1; }();
       const size_t row_len = p.first ? (N >> p.s) : ((size_t)1 << p.lo);
       const size_t rows = p.first ? (p.n_src / row_len) : (N >> p.lo);
-      if (use_tma && p.s >= 2 && (!p.first || (p.n_src % row_len == 0 && rows >= 1)) && ((uintptr_t)in % 16 == 0)) {
+      if (use_tma && !p.src_tab && p.s >= 2 && (!p.first || (p.n_src % row_len == 0 && rows >= 1)) && ((uintptr_t)in % 16 == 0)) {
         NttTma tma;
         const unsigned rpb = (1u << p.s) < 256u ? (1u << p.s) : 256u;
         if (encode_pass_map(tma, in, row_len, rows, batch, in_stride, p.c, rpb)) {
@@ -560,12 +562,13 @@ size_t trp_ntt_passes(unsigned log_n) { return log_n == 0 ? 1 : (log_n + S_MAX -
 
 int trp_ntt_impl(trp_ctx* ctx, int field, const void* d_src, void* d_dst, size_t batch, unsigned log_n,
                  const uint64_t omega[4], size_t src_stride, size_t dst_stride, unsigned n_src, const void* d_pre,
-                 unsigned pre_period, const void* d_post, unsigned post_period, unsigned n_dst, void* d_tmp) {
+                 unsigned pre_period, const void* d_post, unsigned post_period, unsigned n_dst, void* d_tmp,
+                 const void* const* d_src_tab) {
   if (field == 0)
     return ntt_run<FpParams>(ctx, d_src, d_dst, batch, log_n, omega, src_stride, dst_stride, n_src, d_pre, pre_period,
-                             d_post, post_period, n_dst, d_tmp);
+                             d_post, post_period, n_dst, d_tmp, d_src_tab);
   return ntt_run<FqParams>(ctx, d_src, d_dst, batch, log_n, omega, src_stride, dst_stride, n_src, d_pre, pre_period,
-                           d_post, post_period, n_dst, d_tmp);
+                           d_post, post_period, n_dst, d_tmp, d_src_tab);
 }
 
 // ---- elementwise glue kernels (K7) ------------------------------------------------------------------------

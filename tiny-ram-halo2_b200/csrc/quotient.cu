@@ -18,6 +18,7 @@
 #include "qlower.h"
 
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 
 using namespace ff;
@@ -197,17 +198,37 @@ int launch_vm(trp_domain* d, const Staged& st, int coset, uint4* d_out, unsigned
   return d->field == 0 ? go(FpParams()) : go(FqParams());
 }
 
-// out[q * n + t] = sum_i A[q][i] * P[i * n + t]   (Q x Q constant matrix applied to every coefficient index)
+constexpr unsigned MAX_QUOTIENT_PARTS = 64;   // = the most cosets a domain has (trp_domain::coset_gen)
+constexpr unsigned COMBINE_Q = 8;             // output pieces per thread (grid.y covers the rest)
+struct PartsShape { unsigned n_parts, q_out, q[MAX_QUOTIENT_PARTS]; };
+
+// out[q * n + t] = sum_p sum_i A_p[q][i] * P_p[i * n + t] over the parts p with q < Q_p: part p holds the remainders of its values
+// on cosets 0 .. Q_p - 1 (P_p[i], rows after those of the earlier parts) and A_p is its Q_p x Q_p constant matrix (the matrices back
+// to back in A).  A thread owns pieces q0 .. q0 + 7 of one coefficient index, kept in registers; each input element it needs is
+// read once.
 template <class PR>
-__global__ void cosets_combine_kernel(const uint4* P, const uint4* A, unsigned Q, size_t n, uint4* out) {
+__global__ void cosets_combine_kernel(const uint4* P, const uint4* A, PartsShape sh, size_t n, uint4* out) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n) return;
-  for (unsigned q = 0; q < Q; ++q) {
-    Fe<PR> acc = fe_mul(fe_load<PR>(P + 2 * t), fe_load_ro<PR>(A + 2 * (size_t)(q * Q)));
-    for (unsigned i = 1; i < Q; ++i)
-      acc = fe_add(acc, fe_mul(fe_load<PR>(P + 2 * (i * n + t)), fe_load_ro<PR>(A + 2 * (size_t)(q * Q + i))));
-    fe_store(out + 2 * (q * n + t), acc);
+  const unsigned q0 = blockIdx.y * COMBINE_Q;
+  Fe<PR> acc[COMBINE_Q];
+#pragma unroll
+  for (unsigned q = 0; q < COMBINE_Q; ++q) acc[q] = fe_zero<PR>();
+  size_t row = 0, a_off = 0;
+  for (unsigned p = 0; p < sh.n_parts; ++p) {
+    const unsigned Q = sh.q[p];
+    if (Q > q0)
+      for (unsigned i = 0; i < Q; ++i) {
+        const Fe<PR> v = fe_load<PR>(P + 2 * ((row + i) * n + t));
+#pragma unroll
+        for (unsigned q = 0; q < COMBINE_Q; ++q)
+          if (q0 + q < Q) acc[q] = fe_add(acc[q], fe_mul(v, fe_load_ro<PR>(A + 2 * (a_off + (q0 + q) * Q + i))));
+      }
+    row += Q; a_off += (size_t)Q * Q;
   }
+#pragma unroll
+  for (unsigned q = 0; q < COMBINE_Q; ++q)
+    if (q0 + q < sh.q_out) fe_store(out + 2 * ((q0 + q) * n + t), acc[q]);
 }
 
 // A' = V^-1 * diag(1 / ((gamma_i - 1) n))  (or diag(1/n) without the vanishing division), V[i][q] = gamma_i^q,
@@ -250,32 +271,38 @@ int build_combine_matrix(trp_domain* d, unsigned Q, int divide, std::vector<Fe<P
 }
 
 template <class PR>
-int cosets_to_coeff_run(trp_domain* d, uint64_t* d_vals, unsigned Q, uint64_t* d_out, int divide) {
+int cosets_to_coeff_run(trp_domain* d, uint64_t* d_vals, const PartsShape& sh, uint64_t* d_out, int divide) {
   trp_ctx* ctx = d->ctx;
   const size_t n = (size_t)1 << d->k;
   std::vector<Fe<PR>> A;
-  TRP_TRY(build_combine_matrix<PR>(d, Q, divide, A));
+  for (unsigned p = 0; p < sh.n_parts; ++p) {
+    std::vector<Fe<PR>> Ap;
+    TRP_TRY(build_combine_matrix<PR>(d, sh.q[p], divide, Ap));
+    A.insert(A.end(), Ap.begin(), Ap.end());
+  }
   const bool need_tmp = trp_ntt_passes(d->k) > 1;
-  const size_t a_bytes = ws_align((size_t)Q * Q * 32);
+  const size_t a_bytes = ws_align(A.size() * 32);
   TRP_TRY(trp_ws_reserve(ctx, a_bytes + (need_tmp ? n * 32 : 0)));
   char* w = (char*)ctx->ws;
-  TRP_CUDA(ctx, cudaMemcpyAsync(w, A.data(), (size_t)Q * Q * 32, cudaMemcpyHostToDevice, ctx->stream));
+  TRP_CUDA(ctx, cudaMemcpyAsync(w, A.data(), A.size() * 32, cudaMemcpyHostToDevice, ctx->stream));
   TRP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // A is a local
-  for (unsigned i = 0; i < Q; ++i) {
-    // P'_i[t] = c_i^-t * iNTT_omega(values)[t]: the coset-i remainder h mod (X^n - gamma_i), up to the factors folded into A
-    uint64_t cinv[4];
-    {
-      Fe<PR> c; for (int l = 0; l < 4; ++l) { c.v[2 * l] = (uint32_t)d->coset_gen[i][l]; c.v[2 * l + 1] = (uint32_t)(d->coset_gen[i][l] >> 32); }
-      Fe<PR> ci = fe_inv(c);
-      for (int l = 0; l < 4; ++l) cinv[l] = (uint64_t)ci.v[2 * l] | ((uint64_t)ci.v[2 * l + 1] << 32);
+  size_t row = 0;
+  for (unsigned p = 0; p < sh.n_parts; ++p)
+    for (unsigned i = 0; i < sh.q[p]; ++i, ++row) {
+      // P'_i[t] = c_i^-t * iNTT_omega(values)[t]: the coset-i remainder h_p mod (X^n - gamma_i), up to the factors folded into A_p
+      uint64_t cinv[4];
+      {
+        Fe<PR> c; for (int l = 0; l < 4; ++l) { c.v[2 * l] = (uint32_t)d->coset_gen[i][l]; c.v[2 * l + 1] = (uint32_t)(d->coset_gen[i][l] >> 32); }
+        Fe<PR> ci = fe_inv(c);
+        for (int l = 0; l < 4; ++l) cinv[l] = (uint64_t)ci.v[2 * l] | ((uint64_t)ci.v[2 * l + 1] << 32);
+      }
+      const void* post = nullptr;
+      TRP_TRY(trp_get_powers(ctx, d->field, d->k + 1, cinv, &post));
+      uint64_t* v = d_vals + 4 * row * n;
+      TRP_TRY(trp_ntt_impl(ctx, d->field, v, v, 1, d->k, d->omega_inv, n, n, (unsigned)n, nullptr, 0, post, (unsigned)n, (unsigned)n,
+                           need_tmp ? w + a_bytes : nullptr));
     }
-    const void* post = nullptr;
-    TRP_TRY(trp_get_powers(ctx, d->field, d->k + 1, cinv, &post));
-    uint64_t* v = d_vals + 4 * (size_t)i * n;
-    TRP_TRY(trp_ntt_impl(ctx, d->field, v, v, 1, d->k, d->omega_inv, n, n, (unsigned)n, nullptr, 0, post, (unsigned)n, (unsigned)n,
-                         need_tmp ? w + a_bytes : nullptr));
-  }
-  cosets_combine_kernel<PR><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((const uint4*)d_vals, (const uint4*)w, Q, n, (uint4*)d_out);
+  cosets_combine_kernel<PR><<<dim3((unsigned)((n + 127) / 128), (sh.q_out + COMBINE_Q - 1) / COMBINE_Q), 128, 0, ctx->stream>>>((const uint4*)d_vals, (const uint4*)w, sh, n, (uint4*)d_out);
   TRP_LAUNCHED(ctx);
   return TRP_OK;
 }
@@ -285,37 +312,46 @@ struct Locked {
   explicit Locked(trp_ctx* c) : g(c->mu) { cudaSetDevice(c->device); }
 };
 
-// lower the caller's program (cached: a prover evaluates one program on j - 1 cosets, proof after proof), encode it for this launch
+// lower the caller's program (cached: a prover evaluates the same few programs on its cosets, proof after proof), encode it for this launch
 // (qlower::stage: slot offsets, column addresses) and put program / constants at the front of the arena.  col_ptrs = the columns'
 // device addresses, or NULL if the caller will upload the columns itself right behind the tables, own_col_bytes apart.
 int stage_tables(trp_domain* d, const uint32_t* program, size_t n_instr, unsigned n_regs, const uint64_t* consts, size_t n_consts,
                  const uint64_t* const* col_ptrs, size_t n_cols, size_t own_col_bytes, size_t extra, Staged* st) {
   trp_ctx* ctx = d->ctx;
-  if (ctx->q_src.size() != n_instr * 4 || ctx->q_src_regs != n_regs || ctx->q_src_consts != n_consts ||
-      memcmp(ctx->q_src.data(), program, n_instr * 16) != 0) {
-    ctx->q_src.clear();
-    if (!qlower::lower(program, n_instr, n_regs, n_consts, ctx->q_low, &ctx->q_low_regs))
+  auto& progs = ctx->q_progs;
+  size_t hit = 0;
+  while (hit < progs.size() && !(progs[hit].src.size() == n_instr * 4 && progs[hit].src_regs == n_regs && progs[hit].src_consts == n_consts &&
+                                 memcmp(progs[hit].src.data(), program, n_instr * 16) == 0))
+    ++hit;
+  if (hit == progs.size()) {
+    trp_ctx::QProgram e;
+    if (!qlower::lower(program, n_instr, n_regs, n_consts, e.low, &e.low_regs))
       TRP_FAIL(ctx, TRP_E_INVALID, "quotient program: column index above %u", qlower::MAX_COLS - 1);
-    ctx->q_src.assign(program, program + n_instr * 4);
-    ctx->q_src_regs = n_regs; ctx->q_src_consts = n_consts;
+    e.src.assign(program, program + n_instr * 4);
+    e.src_regs = n_regs; e.src_consts = n_consts;
+    if (progs.size() == 16) progs.pop_back();
+    progs.insert(progs.begin(), std::move(e));
+  } else if (hit > 0) {
+    std::rotate(progs.begin(), progs.begin() + hit, progs.begin() + hit + 1);
   }
+  const trp_ctx::QProgram& q = progs.front();
   unsigned threads, bd_log;
-  if (!vm_geometry(ctx->q_low_regs, &threads, &bd_log))
-    TRP_FAIL(ctx, TRP_E_INVALID, "quotient program needs %u registers (max %u)", ctx->q_low_regs, 200 * 1024 / (32 * 32));
-  const size_t low_bytes = ctx->q_low.size() * 4;                     // includes the trailing NOPs
+  if (!vm_geometry(q.low_regs, &threads, &bd_log))
+    TRP_FAIL(ctx, TRP_E_INVALID, "quotient program needs %u registers (max %u)", q.low_regs, 200 * 1024 / (32 * 32));
+  const size_t low_bytes = q.low.size() * 4;                          // includes the trailing NOPs
   size_t b_prog = ws_align(low_bytes), b_c = ws_align((n_consts + 1) * 32);   // + zeta
   TRP_TRY(trp_ws_reserve(ctx, b_prog + b_c + extra));
   char* w = (char*)ctx->ws;
   std::vector<uint64_t> addr(n_cols ? n_cols : 1);
   for (size_t c = 0; c < n_cols; ++c) addr[c] = col_ptrs ? (uint64_t)(uintptr_t)col_ptrs[c] : (uint64_t)(uintptr_t)(w + b_prog + b_c + c * own_col_bytes);
-  if (!qlower::stage(ctx->q_low, ctx->q_low_regs, bd_log, addr.data(), n_cols, ctx->q_staged))
+  if (!qlower::stage(q.low, q.low_regs, bd_log, addr.data(), n_cols, ctx->q_staged))
     TRP_FAIL(ctx, TRP_E_INVALID, "quotient program: a rotation beyond +-32767 rows or too many registers");
   TRP_CUDA(ctx, cudaMemcpyAsync(w, ctx->q_staged.data(), low_bytes, cudaMemcpyHostToDevice, ctx->stream));
   if (n_consts) TRP_CUDA(ctx, cudaMemcpyAsync(w + b_prog, consts, n_consts * 32, cudaMemcpyHostToDevice, ctx->stream));
   TRP_CUDA(ctx, cudaMemcpyAsync(w + b_prog + n_consts * 32, d->g_coset, 32, cudaMemcpyHostToDevice, ctx->stream));   // consts[n_consts] = zeta
   // the host arrays may be reused by the caller as soon as we return
   TRP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  st->prog = (const uint4*)w; st->n_instr = ctx->q_low.size() / 4 - qlower::PAD; st->n_regs = ctx->q_low_regs;
+  st->prog = (const uint4*)w; st->n_instr = q.low.size() / 4 - qlower::PAD; st->n_regs = q.low_regs;
   st->consts = (const uint4*)(w + b_prog);
   st->after = w + b_prog + b_c;
   return TRP_OK;
@@ -417,6 +453,26 @@ int trp_dev_coeff_to_coset(trp_domain* d, const uint64_t* d_coeff, uint64_t* d_o
   return TRP_OK;
 }
 
+// The same for columns scattered in memory: d_src_tab is a DEVICE array of batch column addresses (n coefficients each), the
+// results go to d_out contiguously (column i at d_out[i * n ..]).  A prover expands on each coset only the columns that the
+// constraints evaluated there read, without copying them together first.
+int trp_dev_coeff_to_coset_gather(trp_domain* d, const uint64_t* const* d_src_tab, uint64_t* d_out, size_t batch, unsigned coset) {
+  if (!d) return TRP_E_INVALID;
+  trp_ctx* ctx = d->ctx;
+  Locked l(ctx);
+  if (batch && (!d_src_tab || !d_out)) TRP_FAIL(ctx, TRP_E_INVALID, "NULL buffer");
+  if (coset >= (1u << (d->ext_k - d->k))) TRP_FAIL(ctx, TRP_E_INVALID, "coset index %u out of range", coset);
+  const size_t n = (size_t)1 << d->k;
+  const void* pw = nullptr;   // (zeta * ext_omega^coset)^i, i < n
+  TRP_TRY(trp_get_powers(ctx, d->field, d->k + 1, d->coset_gen[coset], &pw));
+  for (size_t b0 = 0; b0 < batch; b0 += 65535) {
+    size_t nb = batch - b0 < 65535 ? batch - b0 : 65535;
+    TRP_TRY(trp_ntt_impl(ctx, d->field, nullptr, d_out + 4 * b0 * n, nb, d->k, d->omega, n, n, (unsigned)n, pw, (unsigned)n, nullptr, 0,
+                         (unsigned)n, nullptr, (const void* const*)(d_src_tab + b0)));
+  }
+  return TRP_OK;
+}
+
 // Recover the n * ncos coefficients of a polynomial of degree < n * ncos from its values on the first ncos size-n cosets
 // (zeta * ext_omega^i) * <omega>, i < ncos: per coset an inverse NTT gives h mod (X^n - gamma_i), and one ncos x ncos
 // constant matrix (inverse Vandermonde in gamma_i = (zeta ext_omega^i)^n) applied per coefficient index undoes the
@@ -424,13 +480,30 @@ int trp_dev_coeff_to_coset(trp_domain* d, const uint64_t* d_coeff, uint64_t* d_o
 // gamma_i - 1 on coset i).  Produces exactly extended_to_coeff(divide_by_vanishing_poly(.)) of the full extended
 // domain while evaluating only ncos = j - 1 of its 2^(ext_k - k) cosets (5 of 8 for the TinyRAM circuit).
 int trp_dev_cosets_to_coeff(trp_domain* d, uint64_t* d_vals, unsigned ncos, uint64_t* d_out_coeff, int divide_by_vanishing) {
+  return trp_dev_cosets_to_coeff_parts(d, d_vals, &ncos, 1, ncos, d_out_coeff, divide_by_vanishing);
+}
+
+// The same for a polynomial given as a SUM of parts h = sum_p h_p, deg h_p < n * ncos[p]: part p brings its values on the first
+// ncos[p] cosets (rows after those of the earlier parts), and the coefficients of all parts are summed into ncos_out pieces of n.
+// Each part is recovered exactly as above (its own ncos[p] x ncos[p] inverse Vandermonde), so a part of low degree is evaluated
+// on fewer cosets, and the sum equals trp_dev_cosets_to_coeff of the whole h on ncos_out cosets coefficient for coefficient.
+int trp_dev_cosets_to_coeff_parts(trp_domain* d, uint64_t* d_vals, const unsigned* ncos, unsigned n_parts, unsigned ncos_out,
+                                  uint64_t* d_out_coeff, int divide_by_vanishing) {
   if (!d) return TRP_E_INVALID;
   trp_ctx* ctx = d->ctx;
   Locked l(ctx);
-  if (!d_vals || !d_out_coeff) TRP_FAIL(ctx, TRP_E_INVALID, "NULL buffer");
-  if (ncos == 0 || ncos > (1u << (d->ext_k - d->k))) TRP_FAIL(ctx, TRP_E_INVALID, "ncos = %u out of range", ncos);
-  return d->field == 0 ? cosets_to_coeff_run<FpParams>(d, d_vals, ncos, d_out_coeff, divide_by_vanishing)
-                       : cosets_to_coeff_run<FqParams>(d, d_vals, ncos, d_out_coeff, divide_by_vanishing);
+  if (!d_vals || !d_out_coeff || !ncos) TRP_FAIL(ctx, TRP_E_INVALID, "NULL buffer");
+  if (n_parts == 0 || n_parts > MAX_QUOTIENT_PARTS) TRP_FAIL(ctx, TRP_E_INVALID, "n_parts = %u out of range (1 .. %u)", n_parts, MAX_QUOTIENT_PARTS);
+  const unsigned t_period = 1u << (d->ext_k - d->k);
+  if (ncos_out == 0 || ncos_out > t_period) TRP_FAIL(ctx, TRP_E_INVALID, "ncos_out = %u out of range", ncos_out);
+  PartsShape sh{};
+  sh.n_parts = n_parts; sh.q_out = ncos_out;
+  for (unsigned p = 0; p < n_parts; ++p) {
+    if (ncos[p] == 0 || ncos[p] > ncos_out) TRP_FAIL(ctx, TRP_E_INVALID, "part %u: ncos = %u out of range (1 .. %u)", p, ncos[p], ncos_out);
+    sh.q[p] = ncos[p];
+  }
+  return d->field == 0 ? cosets_to_coeff_run<FpParams>(d, d_vals, sh, d_out_coeff, divide_by_vanishing)
+                       : cosets_to_coeff_run<FqParams>(d, d_vals, sh, d_out_coeff, divide_by_vanishing);
 }
 
 }  // extern "C"

@@ -489,6 +489,125 @@ def eval_ast_at_point(B, ast, polys, x):
         sys.setrecursionlimit(old)
 
 
+def quotient_constraints(cs: ConstraintSystem, cs_degree: int, p: int, delta: int, theta_: int, beta_: int, gamma_: int):
+    """every constraint of the vanishing argument as a poly::Ast over symbolic leaves, in halo2's order: (exprs, leaf keys in
+    leaf-index order).  Its SHAPE depends on the constraint system only; the challenges enter as constants."""
+    leaves, keys = {}, []
+    bf, chunk_len = cs.blinding_factors(), cs_degree - 2
+
+    def leaf(key):
+        if key not in leaves:
+            leaves[key] = len(keys)
+            keys.append(key)
+        return P.Poly(leaves[key], 0)
+
+    def to_ast(e):
+        if isinstance(e, Constant): return P.ConstantTerm(e.value % p)
+        if isinstance(e, Query): return leaf((e.kind, e.column)).with_rotation(e.rotation)
+        if isinstance(e, Negated): return -to_ast(e.a)
+        if isinstance(e, Sum): return to_ast(e.a) + to_ast(e.b)
+        if isinstance(e, Product): return to_ast(e.a) * to_ast(e.b)
+        return to_ast(e.a) * (e.scalar % p)
+
+    l0, l_blind, l_last = leaf("l0"), leaf("l_blind"), leaf("l_last")
+    one = P.ConstantTerm(1)
+    active = one - (l_last + l_blind)
+    exprs = [to_ast(g) for g in cs.gates]
+    if cs.permutation:                          # one grand product per chunk of chunk_len columns
+        zs = [leaf(("perm_z", i)) for i in range(-(-len(cs.permutation) // chunk_len))]
+        exprs.append(l0 * (one - zs[0]))
+        exprs.append(l_last * (zs[-1] * zs[-1] - zs[-1]))
+        for i in range(1, len(zs)):
+            exprs.append(l0 * (zs[i] - zs[i - 1].with_rotation(-(bf + 1))))
+        for i, z in enumerate(zs):
+            cols = cs.permutation[i * chunk_len:(i + 1) * chunk_len]
+            left, right = z.with_rotation(1), z
+            cur_delta = beta_ * pow(delta, i * chunk_len, p) % p
+            for off, (kk, c) in enumerate(cols):
+                col = leaf((kk, c))
+                sig = leaf(("sigma", i * chunk_len + off))
+                left = left * (col + sig * beta_ + gamma_)
+                right = right * (col + P.LinearTerm(cur_delta) + gamma_)
+                cur_delta = cur_delta * delta % p
+            exprs.append((left - right) * active)
+    for li, (inputs, tables) in enumerate(cs.lookups):
+        z, a, s = leaf(("lookup_z", li)), leaf(("lookup_a", li)), leaf(("lookup_s", li))
+        comp = lambda es: P.DistributePowers([to_ast(e) for e in es], P.ConstantTerm(theta_)) if len(es) > 1 else to_ast(es[0])
+        exprs.append(l0 * (one - z))
+        exprs.append(l_last * (z * z - z))
+        exprs.append((z.with_rotation(1) * (a + beta_) * (s + gamma_) - z * (comp(inputs) + beta_) * (comp(tables) + gamma_)) * active)
+        exprs.append(l0 * (a - s))
+        exprs.append(((a - s) * (a - a.with_rotation(-1))) * active)
+    return exprs, keys
+
+
+def ast_degree(ast, memo=None) -> int:
+    """upper bound on the degree in X of an Ast whose leaves have degree < n, in units of n (halo2's bound: a leaf and X count 1)"""
+    memo = {} if memo is None else memo
+    key = id(ast)
+    if key not in memo:
+        if isinstance(ast, (P.Poly, P.LinearTerm)): d = 1
+        elif isinstance(ast, P.ConstantTerm): d = 0
+        elif isinstance(ast, P.Add): d = max(ast_degree(ast.a, memo), ast_degree(ast.b, memo))
+        elif isinstance(ast, P.Mul): d = ast_degree(ast.a, memo) + ast_degree(ast.b, memo)
+        elif isinstance(ast, P.Scale): d = ast_degree(ast.a, memo)
+        elif isinstance(ast, P.DistributePowers): d = max([ast_degree(ast.base, memo) * (len(ast.terms) - 1)] + [ast_degree(t, memo) for t in ast.terms])
+        else: raise TypeError(type(ast))
+        memo[key] = d
+    return memo[key]
+
+
+def split_by_degree(exprs, keys, y, cs_degree, p):
+    """The folded numerator N = sum_i y^(m-1-i) exprs[i] as parts N_d, one per degree bound d of the constraints: every expr
+    vanishes on the domain by itself, so h_d = N_d / (X^n - 1) has degree < (d - 1) n and needs only d - 1 cosets, and sum_d h_d is
+    the quotient h.  Returns [(d - 1, Ast, leaf keys)] by increasing d; each part keeps its terms' powers of y (y^gap constants
+    between its terms) and numbers its own leaves.  Degrees below 2 join d = 2 (a degree-1 numerator that vanishes on the
+    domain is zero); a bound above cs_degree would break the monolithic quotient too, and raises."""
+    memo = {}
+    groups = {}
+    for i, e in enumerate(exprs):
+        d = max(ast_degree(e, memo), 2)
+        if d > cs_degree:
+            raise ValueError(f"constraint {i} has degree {d} > the constraint system's degree {cs_degree}")
+        groups.setdefault(d, []).append(i)
+    m, out = len(exprs), []
+    for d in sorted(groups):
+        acc, last = None, None
+        for i in groups[d]:
+            e = exprs[i]
+            acc = e if acc is None else acc * P.ConstantTerm(pow(y, i - last, p)) + e
+            last = i
+        if m - 1 - last:
+            acc = acc * P.ConstantTerm(pow(y, m - 1 - last, p))
+        local, rebuilt = {}, {}
+
+        def remap(a):                       # the part's own leaf numbering; shared subtrees stay shared (x * x stays a square)
+            r = rebuilt.get(id(a))
+            if r is not None:
+                return r
+            if isinstance(a, P.Poly):
+                r = P.Poly(local.setdefault(a.index, len(local)), a.rotation)
+            elif isinstance(a, (P.Add, P.Mul)):
+                r = type(a)(remap(a.a), remap(a.b))
+            elif isinstance(a, P.Scale):
+                r = P.Scale(remap(a.a), a.scalar)
+            elif isinstance(a, P.DistributePowers):
+                r = P.DistributePowers([remap(t) for t in a.terms], remap(a.base))
+            else:
+                r = a
+            rebuilt[id(a)] = r
+            return r
+
+        import sys
+        old = sys.getrecursionlimit(); sys.setrecursionlimit(max(old, 100000))
+        try:
+            ast = remap(acc)
+        finally:
+            sys.setrecursionlimit(old)
+        out.append((d - 1, ast, [keys[g] for g in sorted(local, key=local.get)]))
+    return out
+
+
 def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], int], transcript: Blake2bWrite, debug: bool = False,
                  timings: Optional[dict] = None) -> bytes:
     """plonk::create_proof for ONE circuit instance.  instances: one column per instance column, advice: one per advice column
@@ -614,60 +733,19 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     # ---- quotient --------------------------------------------------------------------------------------------------------------------
     y = transcript.squeeze_challenge_scalar()
     cos_of = {ADVICE: adv_cosets, FIXED: pk.fixed_cosets, INSTANCE: inst_cosets}
-    n_lookups = len(lookups)
 
     def build_h(theta_, beta_, gamma_, y_):
-        """the folded constraint polynomial as a poly::Ast over symbolic leaves: (h_ast, leaf keys in leaf-index order).  Its SHAPE
-        depends on the constraint system only; the challenges enter as constants."""
-        leaves, keys = {}, []
-
-        def leaf(key):
-            if key not in leaves:
-                leaves[key] = len(keys)
-                keys.append(key)
-            return P.Poly(leaves[key], 0)
-
-        def to_ast(e):
-            if isinstance(e, Constant): return P.ConstantTerm(e.value % p)
-            if isinstance(e, Query): return leaf((e.kind, e.column)).with_rotation(e.rotation)
-            if isinstance(e, Negated): return -to_ast(e.a)
-            if isinstance(e, Sum): return to_ast(e.a) + to_ast(e.b)
-            if isinstance(e, Product): return to_ast(e.a) * to_ast(e.b)
-            return to_ast(e.a) * (e.scalar % p)
-
-        l0, l_blind, l_last = leaf("l0"), leaf("l_blind"), leaf("l_last")
-        one = P.ConstantTerm(1)
-        active = one - (l_last + l_blind)
-        exprs = [to_ast(g) for g in cs.gates]
-        if perm_sets:
-            zs = [leaf(("perm_z", i)) for i in range(len(perm_sets))]
-            exprs.append(l0 * (one - zs[0]))
-            exprs.append(l_last * (zs[-1] * zs[-1] - zs[-1]))
-            for i in range(1, len(zs)):
-                exprs.append(l0 * (zs[i] - zs[i - 1].with_rotation(-(bf + 1))))
-            for i, z in enumerate(zs):
-                cols = cs.permutation[i * chunk_len:(i + 1) * chunk_len]
-                left, right = z.with_rotation(1), z
-                cur_delta = beta_ * pow(B.delta, i * chunk_len, p) % p
-                for off, (kk, c) in enumerate(cols):
-                    col = leaf((kk, c))
-                    sig = leaf(("sigma", i * chunk_len + off))
-                    left = left * (col + sig * beta_ + gamma_)
-                    right = right * (col + P.LinearTerm(cur_delta) + gamma_)
-                    cur_delta = cur_delta * B.delta % p
-                exprs.append((left - right) * active)
-        for li, (inputs, tables) in enumerate(cs.lookups[:n_lookups]):
-            z, a, s = leaf(("lookup_z", li)), leaf(("lookup_a", li)), leaf(("lookup_s", li))
-            comp = lambda es: P.DistributePowers([to_ast(e) for e in es], P.ConstantTerm(theta_)) if len(es) > 1 else to_ast(es[0])
-            exprs.append(l0 * (one - z))
-            exprs.append(l_last * (z * z - z))
-            exprs.append((z.with_rotation(1) * (a + beta_) * (s + gamma_) - z * (comp(inputs) + beta_) * (comp(tables) + gamma_)) * active)
-            exprs.append(l0 * (a - s))
-            exprs.append(((a - s) * (a - a.with_rotation(-1))) * active)
+        """the folded constraint polynomial sum_i y^(m-1-i) expr_i as one Ast: (h_ast, leaf keys)"""
+        exprs, keys = quotient_constraints(cs, vk.cs_degree, p, B.delta, theta_, beta_, gamma_)
         h = P.ConstantTerm(0)
         for e in exprs:
             h = h * y_ + e
         return h, keys
+
+    def build_parts(theta_, beta_, gamma_, y_):
+        """the same sum split by constraint degree (quotient_parts)"""
+        exprs, keys = quotient_constraints(cs, vk.cs_degree, p, B.delta, theta_, beta_, gamma_)
+        return split_by_degree(exprs, keys, y_, vk.cs_degree, p)
 
     def resolve(key):                           # the polynomial of THIS proof behind a leaf key
         if isinstance(key, str):
@@ -686,17 +764,26 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     # A backend may keep the compiled program of a proving key (its code depends on the constraint system only) and patch the
     # challenge-dependent constants: GpuBackend.quotient_program.  h_ast itself is then built only for debug.
     h_ast = None
-    cached = getattr(B, "quotient_program", None)
-    prog_and_keys = cached(pk, build_h, (theta, beta, gamma, y), len(cs.permutation)) if cached is not None else None
-    if prog_and_keys is not None:
-        h_in, keys = prog_and_keys
+    challenges = (theta, beta, gamma, y)
+    by_parts = getattr(B, "quotient_parts", None)
+    if by_parts is not None:           # one program per constraint degree, each evaluated on the cosets its degree needs
+        parts = B.quotient_part_programs(pk, build_parts, challenges, len(cs.permutation))
+        pieces = by_parts([(ncos, prog, [resolve(k_) for k_ in pkeys]) for ncos, prog, pkeys in parts])
+        if debug:
+            h_ast, keys = build_h(*challenges)
+            ext_polys = [resolve(k_) for k_ in keys]
     else:
-        h_ast, keys = build_h(theta, beta, gamma, y)
-        h_in = h_ast
-    ext_polys = [resolve(k_) for k_ in keys]
-    if debug and h_ast is None:
-        h_ast, _ = build_h(theta, beta, gamma, y)
-    pieces = B.quotient(h_in, ext_polys)                        # the j - 1 pieces (n coefficients each) of h(X)
+        cached = getattr(B, "quotient_program", None)
+        prog_and_keys = cached(pk, build_h, challenges, len(cs.permutation)) if cached is not None else None
+        if prog_and_keys is not None:
+            h_in, keys = prog_and_keys
+        else:
+            h_ast, keys = build_h(*challenges)
+            h_in = h_ast
+        ext_polys = [resolve(k_) for k_ in keys]
+        if debug and h_ast is None:
+            h_ast, _ = build_h(*challenges)
+        pieces = B.quotient(h_in, ext_polys)                    # the j - 1 pieces (n coefficients each) of h(X)
     if debug:        # h(X) (X^n - 1) must equal the folded constraint polynomial: checked at a point outside the domain
         if not getattr(B, "leaves_are_coefficients", False):
             raise ValueError("debug=True needs a backend whose quotient leaves stay in coefficient form (GpuBackend)")
@@ -1217,76 +1304,117 @@ class GpuBackend:
         evaluate the formulas (microseconds) instead of rebuilding and recompiling the Ast (~60 ms of Python at 8 000
         instructions, during which the GPU would idle: the challenge y is the last thing the transcript yields before the
         quotient).  Any slot that cannot be explained disables the cache for that key."""
+        return GpuBackend._cached_program(self, pk, id(self), build_h, challenges, n_perm_columns)   # self may be another backend (tests)
+
+    def quotient_part_programs(self, pk, build_parts, challenges, n_perm_columns):
+        """[(ncos, Program, leaf keys)] of create_proof's build_parts: one program per constraint degree, each cached like the
+        whole one (a part's constants may also be powers of y); a part the cache cannot explain is compiled afresh"""
+        built = {}
+
+        def parts_at(ch):
+            if ch not in built:
+                built[ch] = build_parts(*ch)
+            return built[ch]
+
+        cache = pk.__dict__.setdefault("_quotient_program", {})
+        shape = cache.get((id(self), "parts"))
+        if shape is None:                         # the degrees depend on the constraint system only
+            shape = cache[(id(self), "parts")] = [ncos for ncos, _, _ in parts_at(tuple(challenges))]
+        out = []
+        for i, ncos in enumerate(shape):
+            got = self._cached_program(pk, (id(self), "part", i), lambda *ch, i=i: parts_at(ch)[i][1:], challenges, n_perm_columns)
+            if got is None:
+                return [(q, P.compile_ast(ast, self.p), keys) for q, ast, keys in parts_at(tuple(challenges))]
+            out.append((ncos, got[0], got[1]))
+        return out
+
+    def _cached_program(self, pk, cache_key, build, challenges, n_perm_columns):
         p = self.p
         cache = pk.__dict__.setdefault("_quotient_program", {})
-        entry = cache.get(id(self))
+        entry = cache.get(cache_key)
         if entry is None:
             real = tuple(c % p for c in challenges)
             probe = tuple((c * 0x9e3779b97f4a7c15 + 0x632be59bd9b4e019 + i) % p for i, c in enumerate(real))
-            ast_r, keys_r = build_h(*real)
-            ast_p, keys_p = build_h(*probe)
+            ast_r, keys_r = build(*real)
+            ast_p, keys_p = build(*probe)
             prog_r, prog_p = P.compile_ast(ast_r, p), P.compile_ast(ast_p, p)
             entry = False
             if keys_r == keys_p and prog_r.code.shape == prog_p.code.shape and (prog_r.code == prog_p.code).all() and len(prog_r.consts) == len(prog_p.consts):
-                def formulas(ch):
+                def formulas(ch, max_gap):
                     theta, beta, gamma, y = ch
                     f = {("theta",): theta, ("beta",): beta, ("gamma",): gamma, ("y",): y}
                     d = beta
                     for i in range(n_perm_columns):
                         f[("beta_delta", i)] = d
                         d = d * self.delta % p
+                    yp = y
+                    for e in range(2, max_gap + 1):             # split_by_degree's y^gap between the terms of a part
+                        yp = yp * y % p
+                        f[("y_pow", e)] = yp
                     return f
-                fr, fp = formulas(real), formulas(probe)
+                fr, fp = formulas(real, 1024), formulas(probe, 1024)
+                by_value = {}
+                for name in fr:
+                    by_value.setdefault((fr[name], fp[name]), name)
                 slots = []
                 for vr, vp in zip(prog_r.consts, prog_p.consts):
                     if vr == vp:
                         slots.append(None)                      # a literal of the constraint system
                         continue
-                    match = [name for name in fr if fr[name] == vr and fp[name] == vp]
-                    if len(match) < 1:
+                    name = by_value.get((vr, vp))
+                    if name is None:
                         slots = None
                         break
-                    slots.append(match[0])
+                    slots.append(name)
                 if slots is not None:
-                    entry = (prog_r, keys_r, slots, formulas)
-            cache[id(self)] = entry
+                    max_gap = max([name[1] for name in slots if name is not None and name[0] == "y_pow"], default=1)
+                    entry = (prog_r, keys_r, slots, formulas, max_gap)
+            cache[cache_key] = entry
             if entry:
                 return entry[0], entry[1]
             return None
         if entry is False:
             return None
-        prog, keys, slots, formulas = entry
-        f = formulas(tuple(c % p for c in challenges))
+        prog, keys, slots, formulas, max_gap = entry
+        f = formulas(tuple(c % p for c in challenges), max_gap)
         consts = [v if name is None else f[name] for v, name in zip(prog.consts, slots)]
         return P.Program(prog.code, consts, prog.n_regs, prog.n_cols), keys
 
-    def quotient(self, ast, ext_polys):
+    def quotient_parts(self, parts):
+        """h(X) from the numerator given by parts [(ncos, Program, leaf polynomials)]: part p is evaluated on cosets 0 .. ncos - 1
+        only, and coset c expands only the coefficient columns that the parts evaluated there read (one gathered batch of NTTs;
+        key material comes from its precomputed cosets).  Columns are numbered by the last coset that needs them, so coset c's
+        columns are a prefix of coset 0's and keep their slot.  Returns the j - 1 pieces of h (n coefficients each)."""
         from ._lib import Q_CONTIGUOUS
-        t, n, ncos = self.torch, self.n, self.j - 1
-        prog = ast if isinstance(ast, P.Program) else P.compile_ast(ast, self.p)
-        dyn = [i for i, c in enumerate(ext_polys) if id(c) not in self._static]
-        in_arena = [self._arena_slot.get(id(ext_polys[i])) for i in dyn]
-        if dyn and all(a is not None and a[1] is ext_polys[i] for a, i in zip(in_arena, dyn)):
-            coeff = self._arena[:self._arena_used]                    # the proof's polynomials, already one contiguous block
-            slot = {i: a[0] for a, i in zip(in_arena, dyn)}
-        else:                                                          # (cols, n, 4) staging copy for the batched coset NTT
-            coeff = t.stack([ext_polys[i] for i in dyn])
-            slot = {i: s_ for s_, i in enumerate(dyn)}
-        ncols = coeff.shape[0]
-        if self._coset_buf is None or self._coset_buf.shape[0] < ncols:      # kept across proofs: a fresh 15.5 GiB block per proof
-            self._coset_buf = None                                           # costs the caching allocator 0.1 s every other proof
-            self._coset_buf = t.empty((ncols, n, 4), dtype=t.int64, device="cuda")
-        buf = self._coset_buf[:ncols]
-        vals = t.empty((ncos, n, 4), dtype=t.int64, device="cuda")
-        self._sync()
-        for cs in range(ncos):
-            self.ctx.check(self.lib.trp_dev_coeff_to_coset(self.dom.handle, coeff.data_ptr(), buf.data_ptr(), ncols, cs))
-            ptrs = [buf[slot[i]].data_ptr() if i in slot else self._static[id(c)][cs].data_ptr() for i, c in enumerate(ext_polys)]
-            self.ev.evaluate_device(prog, self.dom, ptrs, vals[cs].data_ptr(), coset=cs | Q_CONTIGUOUS)
-        h = t.empty((ncos, n, 4), dtype=t.int64, device="cuda")
-        self.ctx.check(self.lib.trp_dev_cosets_to_coeff(self.dom.handle, vals.data_ptr(), ncos, h.data_ptr(), 1))
-        self._sync()
-        return [h[i] for i in range(ncos)]
+        t, n, ncos_out = self.torch, self.n, self.j - 1
+        last = {}                                  # id -> (last coset + 1, polynomial) of every column transformed here
+        for ncos, _, polys in parts:
+            for c in polys:
+                if id(c) not in self._static and last.get(id(c), (0,))[0] < ncos:
+                    last[id(c)] = (ncos, c)
+        order = sorted(last.values(), key=lambda e: -e[0])                # stable: first-use order within a coset count
+        slot = {id(c): s_ for s_, (_, c) in enumerate(order)}
+        count = [sum(1 for q, _ in order if q > cs) for cs in range(ncos_out)]
+        tab = t.tensor([c.data_ptr() for _, c in order] or [0], dtype=t.int64).cuda()
+        if self._coset_buf is None or self._coset_buf.shape[0] < len(order):   # kept across proofs: a fresh 15.5 GiB block per proof
+            self._coset_buf = None                                              # costs the caching allocator 0.1 s every other proof
+            self._coset_buf = t.empty((max(len(order), 1), n, 4), dtype=t.int64, device="cuda")
+        buf = self._coset_buf
+        row = [0]
+        for ncos, _, _ in parts:
+            row.append(row[-1] + ncos)
+        vals = t.empty((row[-1], n, 4), dtype=t.int64, device="cuda")
+        for cs in range(ncos_out):
+            if count[cs]:
+                self.ctx.check(self.lib.trp_dev_coeff_to_coset_gather(self.dom.handle, tab.data_ptr(), buf.data_ptr(), count[cs], cs))
+            for pi, (ncos, prog, polys) in enumerate(parts):
+                if cs < ncos:
+                    ptrs = [buf[slot[id(c)]].data_ptr() if id(c) in slot else self._static[id(c)][cs].data_ptr() for c in polys]
+                    self.ev.evaluate_device(prog, self.dom, ptrs, vals[row[pi] + cs].data_ptr(), coset=cs | Q_CONTIGUOUS)
+        h = t.empty((ncos_out, n, 4), dtype=t.int64, device="cuda")
+        qs = (self.ct.c_uint * len(parts))(*[ncos for ncos, _, _ in parts])
+        self.ctx.check(self.lib.trp_dev_cosets_to_coeff_parts(self.dom.handle, vals.data_ptr(), qs, len(parts), ncos_out, h.data_ptr(), 1))
+        return [h[i] for i in range(ncos_out)]
 
     def eval_polynomial(self, v, x):
         out = self._new(1)

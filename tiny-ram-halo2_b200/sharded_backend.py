@@ -372,10 +372,14 @@ class ShardedGpuBackend(ShardedCommits, GpuBackend):
         return c
 
     # -- the quotient: NTTs by column block, program by row slice --------------------------------------------------------------------------
+    @property
+    def quotient_parts(self):
+        """one GPU: GpuBackend.quotient_parts (the numerator split by constraint degree); several: None, and create_proof hands the
+        whole program to quotient() below"""
+        return super().quotient_parts if self.world == 1 else None
+
     def quotient(self, ast, ext_polys):
         self._drain()
-        if self.world == 1:
-            return super().quotient(ast, ext_polys)
         t, n, ncos, G, H = self.torch, self.n, self.j - 1, self.world, self.HALO
         dyn = [i for i, c in enumerate(ext_polys) if id(c) not in self._static]
         in_arena = [self._arena_slot.get(id(ext_polys[i])) for i in dyn]
