@@ -9,8 +9,9 @@ TEST INFRASTRUCTURE ONLY (see pasta_model.py's header): the product never import
                       plonk.Expression), its own point-set construction.  A proof it accepts satisfies every identity of the
                       protocol at the challenge points, which pins commitments, quotient, evaluations, multiopen and the IPA
                       TOGETHER (the reference's own tests check exactly this accept/reject bit).
-  * PythonBackend     the backend interface of tiny-ram-halo2_b200/plonk.py over pasta_model / params_model, so that the tests can
-                      run the SAME host protocol logic on the CPU and compare proof bytes with the GPU backend's.
+  * PythonBackend     the whole backend interface of tiny-ram-halo2_b200/plonk.py (BACKEND_METHODS) over pasta_model /
+                      params_model, so that the tests can run the SAME host protocol logic on the CPU and compare proof bytes
+                      with the GPU backend's.  Each batch method is the loop over its single-item operation.
 PARITY UNPINNED against a Rust run (no halo2 golden proof exists in /root/reference); see plonk.py's header for the one
 known deviation (transcript_repr)."""
 from __future__ import annotations
@@ -23,6 +24,8 @@ import params_model as prm
 
 # ---- backend for plonk.create_proof / keygen --------------------------------------------------------------------------------------
 class PythonBackend:
+    leaves_are_coefficients = False     # the quotient's leaves are evaluations on the extended domain
+
     def __init__(self, curve: pm.Curve, k: int, cs_degree: int, params=None):
         self.C, self.F = curve, curve.scalar
         self.k, self.n, self.j = k, 1 << k, cs_degree
@@ -44,6 +47,10 @@ class PythonBackend:
     def set_rows(self, v, start, values):
         v[start:start + len(values)] = [x % self.p for x in values]
         return v
+
+    def set_rows_many(self, vs, start, values):
+        for v, vals in zip(vs, values):
+            self.set_rows(v, start, vals)
 
     def random_vec(self, rand): return [rand() for _ in range(self.n)]
 
@@ -67,6 +74,13 @@ class PythonBackend:
             out[i][j] = dl[i2] * om[j2] % p
         return out
 
+    def sigma_swap_blocks(self, sigmas, blocks):
+        for i, r, i2, r2, rows in blocks:
+            for t in range(rows):
+                sigmas[i][r + t] = self.rotate_omega(pow(self.delta, i2, self.p), r2 + t)
+                sigmas[i2][r2 + t] = self.rotate_omega(pow(self.delta, i, self.p), r + t)
+        return sigmas
+
     def compress(self, exprs, theta, values_of):
         p, n = self.p, self.n
         out = [0] * n
@@ -81,11 +95,21 @@ class PythonBackend:
     def commit(self, coeffs, blind):
         return self.C.best_multiexp(list(coeffs) + [blind], self.params["g"] + [self.params["w"]])
 
-    def commit_lagrange_many(self, vecs, blinds): return [self.commit_lagrange(v, b) for v, b in zip(vecs, blinds)]
+    def commit_lagrange_many(self, vecs, blinds, sparse=False, runs=False): return [self.commit_lagrange(v, b) for v, b in zip(vecs, blinds)]
     def commit_many(self, vecs, blinds): return [self.commit(v, b) for v, b in zip(vecs, blinds)]
 
     def lagrange_to_coeff(self, values): return self.dom.lagrange_to_coeff(list(values))
+    def lagrange_to_coeff_many(self, vs): return [self.lagrange_to_coeff(v) for v in vs]
     def coeff_to_extended(self, coeffs): return self.dom.coeff_to_extended(list(coeffs))
+    def coeff_to_extended_static(self, coeffs): return self.coeff_to_extended(coeffs)
+
+    def begin_proof(self, n_polys): pass
+    def end_proof(self): pass
+    def _wait(self): pass
+
+    def quotient_pieces(self, pk, challenges, build_h, build_parts, resolve):
+        ast, keys = build_h(*challenges)                # the whole folded numerator
+        return self.quotient(ast, [resolve(k) for k in keys])
 
     def quotient(self, ast, ext_polys):
         h = pm.evaluate_ast(self.dom, ast, ext_polys)
@@ -93,6 +117,8 @@ class PythonBackend:
         return [h[i * self.n:(i + 1) * self.n] for i in range(self.j - 1)]
 
     def eval_polynomial(self, coeffs, x): return pm.eval_polynomial(self.F, coeffs, x)
+    def eval_polynomials_at(self, vs, x): return [self.eval_polynomial(v, x) for v in vs]
+    def linear_combination(self, vs, scalars): return [sum(s * c for s, c in zip(scalars, col)) % self.p for col in zip(*vs)]
     def kate_division(self, coeffs, b): return pm.kate_division(self.F, list(coeffs), b) + [0]
 
     def permutation_commit(self, values, sigmas, beta, gamma, chunk_len, blinding_factors, rand, after_chunk):
@@ -106,6 +132,23 @@ class PythonBackend:
 
     def lookup_product(self, ci, ct, pi, pt, beta, gamma, blinding_factors, rand):
         return pm.lookup_commit_product(self.F, self.n, ci, ct, pi, pt, beta, gamma, blinding_factors, rand)
+
+    def lookups_commit_permuted(self, lookups, theta, values_of, usable, bf, rand):
+        """lookup::Argument::commit_permuted for each lookup in turn: A' and S' get their blinding rows, then their two blinds"""
+        out = []
+        for inputs, tables in lookups:
+            ci, ct = self.compress(inputs, theta, values_of), self.compress(tables, theta, values_of)
+            pi, pt = self.permute_expression_pair(ci, ct, usable)
+            self.set_rows(pi, usable, [rand() for _ in range(bf + 1)])
+            self.set_rows(pt, usable, [rand() for _ in range(bf + 1)])
+            out.append({"ci": ci, "ct": ct, "pi": pi, "pt": pt, "pi_blind": rand(), "pt_blind": rand()})
+        return out
+
+    def lookup_products(self, lookups, beta, gamma, bf, rand):
+        """Permuted::commit_product for each lookup in turn: Z with its blinding rows, then its blind"""
+        for L in lookups:
+            L["z"] = self.lookup_product(L["ci"], L["ct"], L["pi"], L["pt"], beta, gamma, bf, rand)
+            L["z_blind"] = rand()
 
     def ipa_create_proof(self, rand, transcript, p_poly, p_blind, x_3):
         pm.ipa_create_proof(self.C, self.k, self.params["g"], self.params["w"], self.params["u"], rand, transcript, list(p_poly), p_blind, x_3)

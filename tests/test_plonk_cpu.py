@@ -188,7 +188,7 @@ def test_copy_blocks_nested_in_a_wide_block_take_the_general_path(PL):
     assert blocks2 == [(2, 5, 3, 5, 4)]
 
 
-def test_cached_quotient_program_equals_a_fresh_compile(PL):
+def test_cached_quotient_program_equals_a_fresh_compile_in_quotient_pieces(PL):
     """GpuBackend.quotient_program keeps the compiled quotient program of a proving key and patches the challenge-dependent
     constants (theta, beta, gamma, y, beta * DELTA^i).  Run here over the oracle's PythonBackend: for two proofs of the same key
     (the second one takes the cached path) the patched program must equal a fresh compile of that proof's Ast, for the small
@@ -210,8 +210,8 @@ def test_cached_quotient_program_equals_a_fresh_compile(PL):
     class Probe(VM.PythonBackend):
         checked = 0
 
-        def quotient_program(self, pk, build_h, challenges, n_perm):
-            got = PL.GpuBackend.quotient_program(self, pk, build_h, challenges, n_perm)
+        def quotient_pieces(self, pk, challenges, build_h, build_parts, resolve):
+            got = PL.GpuBackend.quotient_program(self, pk, build_h, challenges, len(pk.vk.cs.permutation))
             assert got is not None
             prog, keys = got
             ast, keys_fresh = build_h(*challenges)
@@ -220,7 +220,7 @@ def test_cached_quotient_program_equals_a_fresh_compile(PL):
             Probe.checked += 1
             if self.stop_after_check:
                 raise Stop()
-            return None                                  # carry on with the Ast path: the proof must still verify
+            return super().quotient_pieces(pk, challenges, build_h, build_parts, resolve)     # the proof must still verify
 
     rnd = random.Random(5)
     rand = lambda: rnd.randrange(C.scalar.p)

@@ -4,7 +4,7 @@ halo2_proofs 0.2.0 @ a95945254dcc, the un-vendored dependency the reference call
 -- SURVEY.md 8(f) row f4: the proof assembly that strings the hot kernels together and produces the serialized proof.
 
 The protocol logic below (phase order, RNG draw order, transcript order, query order, point-set construction) is host code,
-as it is in the reference; every piece of field / group arithmetic goes through a BACKEND object:
+as it is in the reference; every piece of field / group arithmetic goes through a BACKEND object (BACKEND_METHODS below):
 
     GpuBackend (this file)      the product: libtrp.so through the ctypes mirrors (commitment / domain / poly / permutation /
                                 lookup / ipa).  There is no CPU fallback; constructing it without a GPU raises TrpError.
@@ -355,12 +355,48 @@ def build_sigmas(cs: ConstraintSystem, n: int, p: int, omega: int, delta: int, c
     return out
 
 
+# ---- the backend interface: all that keygen and create_proof ask of a backend, and every backend implements all of it --------------
+# (GpuBackend, sharded_backend.ShardedGpuBackend, oracle/plonk_model.PythonBackend).  A batch method means the loop over its
+# single-item operation; v is a vector of n values, bf the number of blinding factors.
+BACKEND_ATTRIBUTES = ("n", "p", "q", "k", "j", "extended_k", "omega", "delta",   # 2^k rows, moduli, cs degree, domain constants
+                      "leaves_are_coefficients")       # the quotient's leaves stay in coefficient form (debug=True needs it)
+BACKEND_METHODS = (
+    "rotate_omega",               # (x, rotation) -> omega^rotation x
+    "vec",                        # (values) -> v, zero-padded to n rows
+    "set_rows",                   # (v, start, values) -> v with v[start : start + len(values)] = values
+    "set_rows_many",              # (vs, start, values): set_rows(vs[i], start, values[i]) for each i
+    "random_vec",                 # (rand) -> a random v
+    "mul_add",                    # (acc, s, v) -> acc s + v (v when acc is None)
+    "sub_low",                    # (v, low) -> v - low on the first len(low) coefficients
+    "sigma_vecs",                 # (m, moved) -> m columns of identity labels delta^i omega^j, moved cells relabelled
+    "sigma_swap_blocks",          # (sigmas, blocks) -> sigmas, each block's two row ranges exchanging their identity labels
+    "commit",                     # (v, blind) -> the commitment over g (coefficient form)
+    "commit_many",                # (vs, blinds) -> [commit]
+    "commit_lagrange_many",       # (vs, blinds, sparse=, runs=) -> commitments over g_lagrange; sparse / runs are density hints
+    "lagrange_to_coeff",          # (v) -> coefficients
+    "lagrange_to_coeff_many",     # (vs) -> [lagrange_to_coeff]
+    "coeff_to_extended",          # (coeffs) -> the quotient's leaf for a proof's polynomial
+    "coeff_to_extended_static",   # (coeffs) -> the same for key material, which the backend may cache
+    "begin_proof",                # (n_polys): a proof starts and will bring n_polys polynomials to coefficient form
+    "end_proof",                  # (): the proof is done (keygen calls it too)
+    "_wait",                      # (): block until the enqueued work has finished (phase timings)
+    "lookups_commit_permuted",    # (lookups, theta, values_of, usable, bf, rand) -> per lookup {ci, ct, pi, pt, pi_blind, pt_blind}
+    "permutation_commit",         # (values, sigmas, beta, gamma, chunk_len, bf, rand, after_chunk): after_chunk(z) per chunk
+    "lookup_products",            # (lookups, beta, gamma, bf, rand): sets each lookup's z and z_blind
+    "quotient_pieces",            # (pk, challenges, build_h, build_parts, resolve) -> the j - 1 pieces of h(X)
+    "eval_polynomial",            # (coeffs, x) -> value
+    "eval_polynomials_at",        # (vs, x) -> [eval_polynomial]
+    "linear_combination",         # (vs, scalars) -> sum_j scalars[j] vs[j]
+    "kate_division",              # (coeffs, b) -> (coeffs - coeffs(b)) / (X - b)
+    "ipa_create_proof",           # (rand, transcript, p_poly, p_blind, x_3): the opening argument
+)
+
+
 def keygen(backend, cs: ConstraintSystem, fixed_values, copies=()) -> ProvingKey:
     """keygen_vk + keygen_pk.  fixed_values: one column per fixed column -- a list of at most n ints (zero-padded) or a
     backend vector."""
     n, p = backend.n, backend.p
-    if hasattr(backend, "end_proof"):
-        backend.end_proof()                    # key material never lives in a proof's polynomial arena
+    backend.end_proof()                        # key material never lives in a proof's polynomial arena
     if n < cs.minimum_rows():
         raise ValueError("NotEnoughRowsAvailable")
     if backend.j != cs.degree():
@@ -369,11 +405,8 @@ def keygen(backend, cs: ConstraintSystem, fixed_values, copies=()) -> ProvingKey
         raise ValueError("one column per fixed column")
     fixed_values = [backend.vec(v) for v in fixed_values]
     fixed_commitments = backend.commit_lagrange_many(fixed_values, [1] * len(fixed_values))          # Blind::default() = 1
-    if hasattr(backend, "sigma_swap_blocks"):     # row-range swaps for the blocks no other constraint touches
-        pairs, blocks = _split_disjoint_blocks(cs, n, list(copies))
-        sigma_values = backend.sigma_swap_blocks(backend.sigma_vecs(len(cs.permutation), permutation_mapping(cs, n, pairs)), blocks)
-    else:
-        sigma_values = backend.sigma_vecs(len(cs.permutation), permutation_mapping(cs, n, copies))
+    pairs, blocks = _split_disjoint_blocks(cs, n, list(copies))     # row-range swaps for the blocks no other constraint touches
+    sigma_values = backend.sigma_swap_blocks(backend.sigma_vecs(len(cs.permutation), permutation_mapping(cs, n, pairs)), blocks)
     permutation_commitments = backend.commit_lagrange_many(sigma_values, [1] * len(sigma_values))
     pt = lambda c: "Identity" if c is None else f"({c[0]:#066x}, {c[1]:#066x})"
     text = (f"PinnedVerificationKey {{ base_modulus: {backend.q:#066x}, scalar_modulus: {p:#066x}, domain: PinnedEvaluationDomain {{ k: {backend.k}, "
@@ -384,7 +417,7 @@ def keygen(backend, cs: ConstraintSystem, fixed_values, copies=()) -> ProvingKey
     fixed_polys = [backend.lagrange_to_coeff(v) for v in fixed_values]
     sigma_polys = [backend.lagrange_to_coeff(v) for v in sigma_values]
     bf = cs.blinding_factors()
-    static = getattr(backend, "coeff_to_extended_static", backend.coeff_to_extended)   # key material: cosets may be cached
+    static = backend.coeff_to_extended_static      # key material: cosets may be cached
     ext = lambda lag: static(backend.lagrange_to_coeff(lag))
     l0 = backend.vec([1])
     l_blind = backend.set_rows(backend.vec([]), n - bf, [1] * bf)
@@ -624,16 +657,14 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     if len(instances) != cs.num_instance or len(advice) != cs.num_advice:
         raise ValueError("InvalidInstances / wrong number of advice columns")
     transcript.common_scalar(vk.transcript_repr)
-    if hasattr(B, "begin_proof"):              # instance + advice + (A', S', Z) per lookup + one Z per permutation chunk
-        chunks = -(-len(cs.permutation) // (vk.cs_degree - 2)) if cs.permutation else 0
-        B.begin_proof(cs.num_instance + cs.num_advice + 3 * len(cs.lookups) + chunks)
+    chunks = -(-len(cs.permutation) // (vk.cs_degree - 2)) if cs.permutation else 0
+    B.begin_proof(cs.num_instance + cs.num_advice + 3 * len(cs.lookups) + chunks)     # instance, advice, (A', S', Z) per lookup, Z per chunk
     import time as _time
     _t = [_time.perf_counter()]
 
     def tick(name):                            # wall-clock per phase; an asynchronous backend is drained first so that the
         if timings is not None:                # time lands in the phase that enqueued the work (a handful of waits per proof)
-            if hasattr(B, "_wait"):
-                B._wait()
+            B._wait()
             now = _time.perf_counter()
             timings[name] = timings.get(name, 0.0) + now - _t[0]
             _t[0] = now
@@ -643,57 +674,37 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
             raise ValueError(f"{what} column longer than the usable rows")
         return B.vec(col)
 
-    # instance / advice / permuted lookup columns are often mostly zero (a circuit that uses a fraction of its rows): backends that
-    # keep a narrow MSM table for such columns take the hint (they check the density themselves)
-    sparse_kw = {"sparse": True} if getattr(B, "accepts_sparse_hint", False) else {}
-    # grand-product columns (and permuted lookup columns with a non-zero default) are constant over the rows a circuit leaves
-    # unused: backends that can commit a column through its row-to-row differences take this hint (GpuBackend._commit_many)
-    runs_kw = {"runs": True} if getattr(B, "accepts_runs_hint", False) else {}
+    # commit_lagrange_many's hints (the backend checks the density itself): sparse = mostly zero (instance / advice / permuted lookup
+    # columns of a circuit that uses a fraction of its rows); runs = constant over the rows a circuit leaves unused (grand products,
+    # permuted lookup columns with a non-zero default), so the row-to-row differences are sparse (GpuBackend._commit_many)
 
     # ---- instance columns: commit (not written, only absorbed) -------------------------------------------------------------
     inst_values = [column(c, "InstanceTooLarge: instance") for c in instances]
-    for cm in B.commit_lagrange_many(inst_values, [1] * len(inst_values), **sparse_kw):
+    for cm in B.commit_lagrange_many(inst_values, [1] * len(inst_values), sparse=True):
         transcript.common_point(cm)
-    to_coeff_many = getattr(B, "lagrange_to_coeff_many", lambda vs: [B.lagrange_to_coeff(v) for v in vs])
-    inst_polys = to_coeff_many(inst_values)
+    inst_polys = B.lagrange_to_coeff_many(inst_values)
     inst_cosets = [B.coeff_to_extended(c) for c in inst_polys]
     tick("instance")
 
     # ---- advice columns --------------------------------------------------------------------------------------------------------
     adv_values = [column(c, "advice") for c in advice]
-    adv_rows = [[rand() for _ in range(usable, n)] for _ in adv_values]
-    if hasattr(B, "set_rows_many"):            # one upload for all columns' blinding rows
-        B.set_rows_many(adv_values, usable, adv_rows)
-    else:
-        for v, rows_ in zip(adv_values, adv_rows):
-            B.set_rows(v, usable, rows_)
+    B.set_rows_many(adv_values, usable, [[rand() for _ in range(usable, n)] for _ in adv_values])
     adv_blinds = [rand() for _ in adv_values]
-    for cm in B.commit_lagrange_many(adv_values, adv_blinds, **sparse_kw):
+    for cm in B.commit_lagrange_many(adv_values, adv_blinds, sparse=True):
         transcript.write_point(cm)
-    adv_polys = to_coeff_many(adv_values)
+    adv_polys = B.lagrange_to_coeff_many(adv_values)
     adv_cosets = [B.coeff_to_extended(c) for c in adv_polys]
     values_of = {ADVICE: adv_values, FIXED: pk.fixed_values, INSTANCE: inst_values}
     tick("advice")
 
     # ---- lookups: commit_permuted -------------------------------------------------------------------------------------------------
     theta = transcript.squeeze_challenge_scalar()
-    lookups = []
-    if hasattr(B, "lookups_commit_permuted"):      # a backend that divides the lookups between devices; same draws in the same order
-        lookups = B.lookups_commit_permuted(cs.lookups, theta, values_of, usable, bf, rand)
-    else:
-        for inputs, tables in cs.lookups:
-            ci, ct = B.compress(inputs, theta, values_of), B.compress(tables, theta, values_of)
-            pi, pt = B.permute_expression_pair(ci, ct, usable)
-            B.set_rows(pi, usable, [rand() for _ in range(bf + 1)])
-            B.set_rows(pt, usable, [rand() for _ in range(bf + 1)])
-            L = {"ci": ci, "ct": ct, "pi": pi, "pt": pt}
-            for name in ("pi", "pt"):
-                L[name + "_blind"] = rand()
-            lookups.append(L)
-    for L, pi_poly, pt_poly in zip(lookups, *[to_coeff_many([L[nm] for L in lookups]) for nm in ("pi", "pt")]):
+    lookups = B.lookups_commit_permuted(cs.lookups, theta, values_of, usable, bf, rand)
+    for L, pi_poly, pt_poly in zip(lookups, *[B.lagrange_to_coeff_many([L[nm] for L in lookups]) for nm in ("pi", "pt")]):
         L["pi_poly"], L["pt_poly"] = pi_poly, pt_poly
     # the commitments do not feed the RNG, so they are computed as one batch and written in halo2's order
-    for cm in B.commit_lagrange_many([L[nm] for L in lookups for nm in ("pi", "pt")], [L[nm + "_blind"] for L in lookups for nm in ("pi", "pt")], **sparse_kw, **runs_kw):
+    for cm in B.commit_lagrange_many([L[nm] for L in lookups for nm in ("pi", "pt")], [L[nm + "_blind"] for L in lookups for nm in ("pi", "pt")],
+                                     sparse=True, runs=True):
         transcript.write_point(cm)
     tick("lookups_permuted")
 
@@ -708,20 +719,15 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
 
     if cs.permutation:
         B.permutation_commit([values_of[kk][c] for kk, c in cs.permutation], pk.sigma_values, beta, gamma, chunk_len, bf, rand, after_chunk)
-    for cm in B.commit_lagrange_many([S["z"] for S in perm_sets], [S["blind"] for S in perm_sets], **runs_kw):
+    for cm in B.commit_lagrange_many([S["z"] for S in perm_sets], [S["blind"] for S in perm_sets], runs=True):
         transcript.write_point(cm)
-    for S, poly in zip(perm_sets, to_coeff_many([S["z"] for S in perm_sets])):
+    for S, poly in zip(perm_sets, B.lagrange_to_coeff_many([S["z"] for S in perm_sets])):
         S["poly"] = poly
         S["coset"] = B.coeff_to_extended(poly)
-    if hasattr(B, "lookup_products"):
-        B.lookup_products(lookups, beta, gamma, bf, rand)
-    else:
-        for L in lookups:
-            L["z"] = B.lookup_product(L["ci"], L["ct"], L["pi"], L["pt"], beta, gamma, bf, rand)
-            L["z_blind"] = rand()
-    for cm in B.commit_lagrange_many([L["z"] for L in lookups], [L["z_blind"] for L in lookups], **runs_kw):
+    B.lookup_products(lookups, beta, gamma, bf, rand)
+    for cm in B.commit_lagrange_many([L["z"] for L in lookups], [L["z_blind"] for L in lookups], runs=True):
         transcript.write_point(cm)
-    for L, poly in zip(lookups, to_coeff_many([L["z"] for L in lookups])):
+    for L, poly in zip(lookups, B.lagrange_to_coeff_many([L["z"] for L in lookups])):
         L["z_poly"] = poly
     tick("grand_products")
 
@@ -761,34 +767,16 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
             return L[name + "_ext"]
         return cos_of[tag][key[1]]
 
-    # A backend may keep the compiled program of a proving key (its code depends on the constraint system only) and patch the
-    # challenge-dependent constants: GpuBackend.quotient_program.  h_ast itself is then built only for debug.
-    h_ast = None
+    # The backend picks the form of the numerator (the whole Ast, or parts by degree) and may keep the compiled programs of a
+    # proving key, whose code depends on the constraint system only (GpuBackend.quotient_program).
     challenges = (theta, beta, gamma, y)
-    by_parts = getattr(B, "quotient_parts", None)
-    if by_parts is not None:           # one program per constraint degree, each evaluated on the cosets its degree needs
-        parts = B.quotient_part_programs(pk, build_parts, challenges, len(cs.permutation))
-        pieces = by_parts([(ncos, prog, [resolve(k_) for k_ in pkeys]) for ncos, prog, pkeys in parts])
-        if debug:
-            h_ast, keys = build_h(*challenges)
-            ext_polys = [resolve(k_) for k_ in keys]
-    else:
-        cached = getattr(B, "quotient_program", None)
-        prog_and_keys = cached(pk, build_h, challenges, len(cs.permutation)) if cached is not None else None
-        if prog_and_keys is not None:
-            h_in, keys = prog_and_keys
-        else:
-            h_ast, keys = build_h(*challenges)
-            h_in = h_ast
-        ext_polys = [resolve(k_) for k_ in keys]
-        if debug and h_ast is None:
-            h_ast, _ = build_h(*challenges)
-        pieces = B.quotient(h_in, ext_polys)                    # the j - 1 pieces (n coefficients each) of h(X)
+    pieces = B.quotient_pieces(pk, challenges, build_h, build_parts, resolve)      # the j - 1 pieces (n coefficients each) of h(X)
     if debug:        # h(X) (X^n - 1) must equal the folded constraint polynomial: checked at a point outside the domain
-        if not getattr(B, "leaves_are_coefficients", False):
+        if not B.leaves_are_coefficients:
             raise ValueError("debug=True needs a backend whose quotient leaves stay in coefficient form (GpuBackend)")
+        h_ast, keys = build_h(*challenges)
         xd = 0x1234567890abcdef1234567890abcdef % p
-        lhs = eval_ast_at_point(B, h_ast, ext_polys, xd)
+        lhs = eval_ast_at_point(B, h_ast, [resolve(k_) for k_ in keys], xd)
         hx, xdn = 0, pow(xd, n, p)
         for piece in reversed(pieces):
             hx = (hx * xdn + B.eval_polynomial(piece, xd)) % p
@@ -807,32 +795,28 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     cache = {}
 
     def ev(poly, point):                       # every opened value is computed once (transcript and multiopen share them)
-        key = (id(poly), point)
-        if key not in cache:
-            cache[key] = B.eval_polynomial(poly, point)
-        return cache[key]
+        return cache[(id(poly), point)]
 
     h_poly, h_blind = None, 0
     for piece, b in zip(reversed(pieces), reversed(h_blinds)):
         h_poly = B.mul_add(h_poly, xn, piece)
         h_blind = (h_blind * xn + b) % p
     x_next, x_inv, x_last = rot(x, 1), rot(x, -1), rot(x, -(bf + 1))
-    many = getattr(B, "eval_polynomials_at", None)
-    if many is not None:       # nothing below feeds the transcript back into x: all openings are computed up front, point by point
-        want = [(polys_of[kind][c], rot(x, r)) for kind in (INSTANCE, ADVICE, FIXED) for c, r in cs.queries[kind]]
-        want += [(random_poly, x), (h_poly, x)] + [(sp, x) for sp in pk.sigma_polys]
-        for i, S in enumerate(perm_sets):
-            want += [(S["poly"], x), (S["poly"], x_next)] + ([(S["poly"], x_last)] if i + 1 < len(perm_sets) else [])
-        for L in lookups:
-            want += [(L["z_poly"], x), (L["z_poly"], x_next), (L["pi_poly"], x), (L["pi_poly"], x_inv), (L["pt_poly"], x)]
-        by_point = {}
-        for poly, pt_ in want:
-            if (id(poly), pt_) not in cache:
-                cache[(id(poly), pt_)] = None
-                by_point.setdefault(pt_, []).append(poly)
-        for pt_, polys_ in by_point.items():
-            for poly, val in zip(polys_, many(polys_, pt_)):
-                cache[(id(poly), pt_)] = val
+    # nothing below feeds the transcript back into x: all openings are computed up front, point by point
+    want = [(polys_of[kind][c], rot(x, r)) for kind in (INSTANCE, ADVICE, FIXED) for c, r in cs.queries[kind]]
+    want += [(random_poly, x), (h_poly, x)] + [(sp, x) for sp in pk.sigma_polys]
+    for i, S in enumerate(perm_sets):
+        want += [(S["poly"], x), (S["poly"], x_next)] + ([(S["poly"], x_last)] if i + 1 < len(perm_sets) else [])
+    for L in lookups:
+        want += [(L["z_poly"], x), (L["z_poly"], x_next), (L["pi_poly"], x), (L["pi_poly"], x_inv), (L["pt_poly"], x)]
+    by_point = {}
+    for poly, pt_ in want:
+        if (id(poly), pt_) not in cache:
+            cache[(id(poly), pt_)] = None
+            by_point.setdefault(pt_, []).append(poly)
+    for pt_, polys_ in by_point.items():
+        for poly, val in zip(polys_, B.eval_polynomials_at(polys_, pt_)):
+            cache[(id(poly), pt_)] = val
     for kind in (INSTANCE, ADVICE, FIXED):
         for c, r in cs.queries[kind]:
             transcript.write_scalar(ev(polys_of[kind][c], rot(x, r)))
@@ -879,21 +863,16 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     x_2 = transcript.squeeze_challenge_scalar()
     cmap, point_sets = construct_intermediate_sets(qs, lambda q: (id(q.poly), q.blind), lambda q: q.point, lambda q: q.eval)
     ns = len(point_sets)
-    q_polys, q_blinds = [None] * ns, [0] * ns
+    q_blinds = [0] * ns
     q_eval_sets = [[0] * len(ps) for ps in point_sets]
-    lincomb = getattr(B, "linear_combination", None)
     members = [[] for _ in range(ns)]
     for cd in cmap:
         s, o = cd["set_index"], cd["commitment"]
-        if lincomb is None:
-            q_polys[s] = B.mul_add(q_polys[s], x_1, o.poly)
         members[s].append(o.poly)
         q_blinds[s] = (q_blinds[s] * x_1 + o.blind) % p
         q_eval_sets[s] = [(a * x_1 + e) % p for a, e in zip(q_eval_sets[s], cd["evals"])]
-    if lincomb is not None:       # q_polys[s] = sum_j x_1^(r - 1 - j) * member_j: the same Horner fold, one pass over the inputs
-        for s, polys_ in enumerate(members):
-            r = len(polys_)
-            q_polys[s] = lincomb(polys_, [pow(x_1, r - 1 - j, p) for j in range(r)])
+    # q_polys[s] = sum_j x_1^(r - 1 - j) * member_j: halo2's Horner fold over the set's members, in one pass over the inputs
+    q_polys = [B.linear_combination(polys_, [pow(x_1, len(polys_) - 1 - j, p) for j in range(len(polys_))]) for polys_ in members]
     q_prime = None
     for points, evals, poly in zip(point_sets, q_eval_sets, q_polys):
         cur = B.sub_low(poly, lagrange_interpolate(points, evals, p))
@@ -913,8 +892,7 @@ def create_proof(backend, pk: ProvingKey, instances, advice, rand: Callable[[], 
     tick("multiopen")
     B.ipa_create_proof(rand, transcript, p_poly, p_blind, x_3)
     tick("ipa")
-    if hasattr(B, "end_proof"):
-        B.end_proof()
+    B.end_proof()
     return transcript.finalize()
 
 
@@ -924,6 +902,7 @@ class GpuBackend:
     limbs in HBM and every operation is a trp_dev_* entry point of include/tr_prover.h; the host sees scalars and points only.
     The quotient is evaluated coset by coset from coefficient form (j - 1 cosets, trp_dev_cosets_to_coeff), so no
     extended-domain column is ever materialised.  No CPU fallback: constructing it without a GPU raises TrpError."""
+    leaves_are_coefficients = True                # coeff_to_extended keeps coefficient form (cosets are expanded in the quotient)
 
     def __init__(self, ctx, k: int, cs_degree: int, params=None):
         import ctypes
@@ -940,9 +919,9 @@ class GpuBackend:
         self.R, self.Rq = (1 << 256) % self.p, (1 << 256) % self.q
         self.Rinv, self.Rqinv = pow(self.R, -1, self.p), pow(self.Rq, -1, self.q)
         # ONE stream for torch's kernels, the library's kernels and NCCL: the ctx is pointed at a torch stream that is made this
-        # thread's current stream, so everything the prover enqueues is ordered by the stream itself and the host only waits
-        # when it reads a result (.cpu()).  (Round 1 kept the library on its own non-blocking stream and fenced every call
-        # with a device-wide synchronize: ~3 000 fences per proof at k = 20.)
+        # thread's current stream, so everything the prover enqueues is ordered by the stream itself: a hand-over between torch
+        # and the library needs no fence, and the host only waits when it reads a result (.cpu()).  (Round 1 kept the library on
+        # its own non-blocking stream and fenced every call with a device-wide synchronize: ~3 000 fences per proof at k = 20.)
         self.stream = ctx.bind_torch_stream()                  # one per process and device, shared by every backend and ctx
         self.params = params if params is not None else Params.new(ctx, k)
         self.dom = EvaluationDomain(ctx, cs_degree, k)
@@ -968,7 +947,6 @@ class GpuBackend:
         if os.environ.get("TRP_COMMIT_BY_PARTS", "1") != "0":
             from .arithmetic import Bases
             d_q = self.torch.from_numpy(np.ascontiguousarray(self.params.g_lagrange_points).view(np.int64)).cuda()
-            self._sync()
             self.ctx.check(self.lib.trp_dev_points_prefix_sum(self.ctx.handle, d_q.data_ptr(), self.n, d_q.data_ptr()))
             q_host = d_q.cpu().numpy().view(np.uint64).reshape(self.n, 8)
             self._gl_prefix = Bases(ctx, np.concatenate([q_host, self.params.w.reshape(1, 8)]), (13 << 8) if k >= 18 else 0)
@@ -977,9 +955,6 @@ class GpuBackend:
         self._static, self._static_keep = {}, []
         self.static_budget_bytes = 48 << 30
         self._arena, self._arena_used, self._arena_slot, self._arena_on, self._coset_buf = None, 0, {}, False, None
-        self.leaves_are_coefficients = True       # coeff_to_extended keeps coefficient form (cosets are expanded in quotient())
-        self.accepts_sparse_hint = True
-        self.accepts_runs_hint = self._gl_prefix is not None
 
     def close(self):
         """release the library-side handles (MSM tables of the opening, the domain); torch tensors follow Python's lifetime"""
@@ -1013,15 +988,10 @@ class GpuBackend:
         f = self.torch.zeros if zero else self.torch.empty
         return f((self.n if rows is None else rows, 4), dtype=self.torch.int64, device="cuda")
 
-    def _sync(self):
-        """kept as the marker of every torch <-> library hand-over; a no-op since both run on self.stream"""
-        return None
-
     def _wait(self):
         self.stream.synchronize()
 
     def _point(self, d_jac):
-        self._sync()
         jac = d_jac.cpu().numpy().view(self.np.uint64).reshape(3, 4)
         if not jac[2].any():
             return None
@@ -1075,32 +1045,25 @@ class GpuBackend:
             return v.clone()
         out = self._new()
         d_s = self._dev(self._limbs([s]))
-        self._sync()
         self.ctx.check(self.lib.trp_dev_field_op(self.ctx.handle, 0, 2 | 16, acc.data_ptr(), d_s.data_ptr(), out.data_ptr(), self.n))
         self.ctx.check(self.lib.trp_dev_field_op(self.ctx.handle, 0, 0, out.data_ptr(), v.data_ptr(), out.data_ptr(), self.n))
-        self._sync()
         return out
 
     def sub_low(self, v, low):
         out = v.clone()
-        self._sync()
         cur = self._ints(out[:len(low)].cpu().numpy().view(self.np.uint64))
         return self.set_rows(out, 0, [(c - r) % self.p for c, r in zip(cur, low)])
 
     def sigma_vecs(self, m, moved):
         base = self._new()
-        self._sync()
         self.ctx.check(self.lib.trp_dev_powers(self.ctx.handle, 0, self._m(self.omega), self.n, base.data_ptr()))
         out, dl = [], 1
         for i in range(m):
             v = self._new()
             d_s = self._dev(self._limbs([dl]))
-            self._sync()
             self.ctx.check(self.lib.trp_dev_field_op(self.ctx.handle, 0, 2 | 16, base.data_ptr(), d_s.data_ptr(), v.data_ptr(), self.n))
-            self._sync()                               # d_s is released below: the kernel reading it must have finished
             out.append(v)
             dl = dl * self.delta % self.p
-        self._sync()
         if moved:                                      # patch the cells the copy constraints move: one scatter per column
             top = max(j2 for _, (_, j2) in moved.items())
             om = [1] * (top + 1)
@@ -1114,7 +1077,6 @@ class GpuBackend:
             for i, (rws, vals) in per_col.items():
                 idx = self.torch.tensor(rws, dtype=self.torch.int64, device="cuda")
                 out[i][idx] = self._dev(self._limbs(vals))
-            self._sync()
         return out
 
     def sigma_swap_blocks(self, sigmas, blocks):
@@ -1123,17 +1085,14 @@ class GpuBackend:
         if not blocks:
             return sigmas
         base = self._new()
-        self._sync()
         self.ctx.check(self.lib.trp_dev_powers(self.ctx.handle, 0, self._m(self.omega), self.n, base.data_ptr()))
         scal = {}
         for (i, r, i2, r2, rows) in blocks:
             for (dst, d0, src, s0) in ((i, r, i2, r2), (i2, r2, i, r)):
                 if src not in scal:
                     scal[src] = self._dev(self._limbs([pow(self.delta, src, self.p)]))
-                self._sync()
                 self.ctx.check(self.lib.trp_dev_field_op(self.ctx.handle, 0, 2 | 16, base[s0:s0 + rows].data_ptr(), scal[src].data_ptr(),
                                                          sigmas[dst][d0:d0 + rows].data_ptr(), rows))
-        self._sync()
         return sigmas
 
     # -- commitments and transforms
@@ -1141,7 +1100,6 @@ class GpuBackend:
         t = self.torch
         stage = t.cat([v, self._dev(self._limbs([blind]))])
         out = t.zeros(12, dtype=t.int64, device="cuda")
-        self._sync()
         self.ctx.check(self.lib.trp_dev_msm_batch(self.ctx.handle, bases.handle, stage.data_ptr(), self.n + 1, 1, out.data_ptr()))
         return self._point(out)
 
@@ -1203,11 +1161,9 @@ class GpuBackend:
         filled = 1
         for u_j in reversed(us):
             d_u = self._dev(self._limbs([u_j]))
-            self._sync()
             self.ctx.check(self.lib.trp_dev_field_op(self.ctx.handle, 0, 2 | 16, s[:filled].data_ptr(), d_u.data_ptr(),
                                                      s[filled:2 * filled].data_ptr(), filled))
             filled *= 2
-        self._sync()
         if filled != self.n:
             raise ValueError("one challenge per round: len(us) must equal k")
         return s
@@ -1220,7 +1176,6 @@ class GpuBackend:
         d_pts = self._dev(self._limbs([c for pt in points for c in pt], self.q, self.Rq).reshape(len(points), 8))
         d_sc = self._dev(self._limbs(scalars))
         out = t.zeros(12, dtype=t.int64, device="cuda")
-        self._sync()
         self.ctx.check(self.lib.trp_dev_msm_var(self.ctx.handle, d_pts.data_ptr(), d_sc.data_ptr(), len(scalars), 1, out.data_ptr()))
         return self._point(out)
 
@@ -1249,9 +1204,7 @@ class GpuBackend:
             c.copy_(v)
         else:
             c = v.clone()
-        self._sync()
         self.ctx.check(self.lib.trp_dev_lagrange_to_coeff(self.dom.handle, c.data_ptr(), 1))
-        self._sync()
         return c
 
     def lagrange_to_coeff_many(self, vs):
@@ -1267,9 +1220,7 @@ class GpuBackend:
             self._arena_used += 1
             c.copy_(v)
             out.append(c)
-        self._sync()
         self.ctx.check(self.lib.trp_dev_lagrange_to_coeff(self.dom.handle, self._arena[first].data_ptr(), k))
-        self._sync()
         return out
 
     def coeff_to_extended(self, c):
@@ -1283,10 +1234,8 @@ class GpuBackend:
         if held + ncos * self.n * 32 > self.static_budget_bytes:
             return c
         vals = self.torch.empty((ncos, self.n, 4), dtype=self.torch.int64, device="cuda")
-        self._sync()
         for cs in range(ncos):
             self.ctx.check(self.lib.trp_dev_coeff_to_coset(self.dom.handle, c.data_ptr(), vals[cs].data_ptr(), 1, cs))
-        self._sync()
         self._static[id(c)] = vals
         self._static_keep.append(c)       # id() stays unique while the tensor is alive
         return c
@@ -1297,7 +1246,7 @@ class GpuBackend:
         self.ev.evaluate_device(prog, self.dom, [c.data_ptr() for c in columns], out.data_ptr(), coset=coset | Q_CONTIGUOUS)
 
     def quotient_program(self, pk, build_h, challenges, n_perm_columns):
-        """The compiled quotient program of `pk` with this proof's challenges patched in, or None (then create_proof builds and
+        """The compiled quotient program of `pk` with this proof's challenges patched in, or None (then the caller builds and
         compiles the Ast as usual).  The program's CODE depends on the constraint system only; its constants are literals of the
         gates or one of theta, beta, gamma, y, beta * DELTA^i.  The first proof of a key compiles the Ast twice -- with the real
         challenges and with a probe set -- and explains every constant slot by exactly one of those formulas; later proofs
@@ -1380,6 +1329,11 @@ class GpuBackend:
         consts = [v if name is None else f[name] for v, name in zip(prog.consts, slots)]
         return P.Program(prog.code, consts, prog.n_regs, prog.n_cols), keys
 
+    def quotient_pieces(self, pk, challenges, build_h, build_parts, resolve):
+        """one program per constraint degree, each evaluated on the cosets its degree needs"""
+        parts = self.quotient_part_programs(pk, build_parts, challenges, len(pk.vk.cs.permutation))
+        return self.quotient_parts([(ncos, prog, [resolve(k_) for k_ in keys]) for ncos, prog, keys in parts])
+
     def quotient_parts(self, parts):
         """h(X) from the numerator given by parts [(ncos, Program, leaf polynomials)]: part p is evaluated on cosets 0 .. ncos - 1
         only, and coset c expands only the coefficient columns that the parts evaluated there read (one gathered batch of NTTs;
@@ -1418,9 +1372,7 @@ class GpuBackend:
 
     def eval_polynomial(self, v, x):
         out = self._new(1)
-        self._sync()
         self.ctx.check(self.lib.trp_dev_eval_polynomials(self.ctx.handle, 0, v.data_ptr(), self.n, self.n, 1, self._m(x), out.data_ptr()))
-        self._sync()
         return self._ints(out.cpu().numpy().view(self.np.uint64))[0]
 
     def eval_polynomials_at(self, vs, x):
@@ -1429,9 +1381,7 @@ class GpuBackend:
             return []
         out = self._new(len(vs))
         tab = (self.ct.c_void_p * len(vs))(*[v.data_ptr() for v in vs])
-        self._sync()
         self.ctx.check(self.lib.trp_dev_eval_polynomials_at(self.ctx.handle, 0, tab, self.n, len(vs), self._m(x), out.data_ptr()))
-        self._sync()
         return self._ints(out.cpu().numpy().view(self.np.uint64))
 
     def linear_combination(self, vs, scalars):
@@ -1439,17 +1389,13 @@ class GpuBackend:
         out = self._new()
         tab = (self.ct.c_void_p * len(vs))(*[v.data_ptr() for v in vs])
         sc = self._limbs(scalars)
-        self._sync()
         from ._lib import ptr
         self.ctx.check(self.lib.trp_dev_linear_combination(self.ctx.handle, 0, tab, ptr(sc), self.n, len(vs), out.data_ptr()))
-        self._sync()
         return out
 
     def kate_division(self, v, b):
         q = self._new(zero=True)
-        self._sync()
         self.ctx.check(self.lib.trp_dev_kate_division(self.ctx.handle, 0, v.data_ptr(), self.n, self._m(b), q.data_ptr()))
-        self._sync()
         return q
 
     # -- lookups and permutation
@@ -1472,19 +1418,15 @@ class GpuBackend:
         for e in exprs:
             ast = ast * theta + to_ast(e)
         out = self._new()
-        self._sync()
         self._run_program(ast, cols, out, 0)          # coset 0, contiguous: rows = n, rotations step by one row
-        self._sync()
         return out
 
     def permute_expression_pair(self, inp, tab, usable_rows):
         from .lookup import ConstraintSystemFailure
         pa, ps = self._new(zero=True), self._new(zero=True)
         ok = self.ct.c_int(1)
-        self._sync()
         self.ctx.check(self.lib.trp_dev_permute_expression_pair(self.ctx.handle, inp.data_ptr(), tab.data_ptr(), usable_rows, pa.data_ptr(),
                                                                 ps.data_ptr(), self.ct.byref(ok)))
-        self._sync()
         if not ok.value:
             raise ConstraintSystemFailure("lookup input value not present in the table")
         return pa, ps
@@ -1500,10 +1442,8 @@ class GpuBackend:
             vptr = (ct.c_void_p * len(cols))(*[values[c].data_ptr() for c in cols])
             sptr = (ct.c_void_p * len(cols))(*[sigmas[c].data_ptr() for c in cols])
             z = self._new()
-            self._sync()
             self.ctx.check(self.lib.trp_dev_permutation_product(self.dom.handle, vptr, sptr, len(cols), self._m(beta), self._m(gamma), ptr(dbeta),
                                                                 None if last is None else last[n - (blinding_factors + 1)].data_ptr(), z.data_ptr()))
-            self._sync()
             self.set_rows(z, n - blinding_factors, [rand() for _ in range(blinding_factors)])
             last = z
             sets.append(z)
@@ -1512,11 +1452,24 @@ class GpuBackend:
 
     def lookup_product(self, ci, ct_, pi, pt, beta, gamma, blinding_factors, rand):
         z = self._new()
-        self._sync()
         self.ctx.check(self.lib.trp_dev_lookup_product(self.dom.handle, ci.data_ptr(), ct_.data_ptr(), pi.data_ptr(), pt.data_ptr(), self._m(beta),
                                                        self._m(gamma), z.data_ptr(), self.n - blinding_factors))
-        self._sync()
         return self.set_rows(z, self.n - blinding_factors, [rand() for _ in range(blinding_factors)])
+
+    def lookups_commit_permuted(self, lookups, theta, values_of, usable, bf, rand):
+        out = []
+        for inputs, tables in lookups:
+            ci, ct_ = self.compress(inputs, theta, values_of), self.compress(tables, theta, values_of)
+            pi, pt = self.permute_expression_pair(ci, ct_, usable)
+            self.set_rows(pi, usable, [rand() for _ in range(bf + 1)])
+            self.set_rows(pt, usable, [rand() for _ in range(bf + 1)])
+            out.append({"ci": ci, "ct": ct_, "pi": pi, "pt": pt, "pi_blind": rand(), "pt_blind": rand()})
+        return out
+
+    def lookup_products(self, lookups, beta, gamma, bf, rand):
+        for L in lookups:
+            L["z"] = self.lookup_product(L["ci"], L["ct"], L["pi"], L["pt"], beta, gamma, bf, rand)
+            L["z_blind"] = rand()
 
     def ipa_create_proof(self, rand, transcript, p_poly, p_blind, x_3):
         outer = self
@@ -1528,7 +1481,6 @@ class GpuBackend:
             def write_scalar(self, s): transcript.write_scalar(s)
             def squeeze_challenge_scalar(self): return transcript.squeeze_challenge_scalar()
 
-        self._sync()
         bulk = (lambda n_: self.random_vec(rand)) if hasattr(rand, "bulk_key") else getattr(rand, "vector", None)
         self._ipa.create_proof(self.ipa_params, rand, _Adapter(), p_poly, p_blind, x_3, rand_vector=bulk, dist=self._ipa_dist())
 

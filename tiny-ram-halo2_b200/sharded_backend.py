@@ -372,11 +372,13 @@ class ShardedGpuBackend(ShardedCommits, GpuBackend):
         return c
 
     # -- the quotient: NTTs by column block, program by row slice --------------------------------------------------------------------------
-    @property
-    def quotient_parts(self):
-        """one GPU: GpuBackend.quotient_parts (the numerator split by constraint degree); several: None, and create_proof hands the
-        whole program to quotient() below"""
-        return super().quotient_parts if self.world == 1 else None
+    def quotient_pieces(self, pk, challenges, build_h, build_parts, resolve):
+        """one GPU: GpuBackend's (the numerator split by constraint degree); several: the whole program, row-sliced by quotient()"""
+        if self.world == 1:
+            return super().quotient_pieces(pk, challenges, build_h, build_parts, resolve)
+        cached = self.quotient_program(pk, build_h, challenges, len(pk.vk.cs.permutation))
+        prog, keys = cached if cached is not None else build_h(*challenges)
+        return self.quotient(prog, [resolve(k_) for k_ in keys])
 
     def quotient(self, ast, ext_polys):
         self._drain()

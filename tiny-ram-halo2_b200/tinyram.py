@@ -903,9 +903,7 @@ def device_columns(be, columns) -> list:
                 v[:, 0] = int(np.uint64(fill).view(np.int64)) if fill >= 1 << 63 else fill
             if len(arr):
                 v[:len(arr), 0] = torch.from_numpy(arr.view(np.int64)).cuda()
-            be._sync()
             be.ctx.check(be.lib.trp_dev_field_op(be.ctx.handle, 0, 2 | 16, v.data_ptr(), r2.data_ptr(), v.data_ptr(), be.n))
-            be._sync()
         else:
             v = be.vec(prefix.tolist() if isinstance(prefix, np.ndarray) else prefix)
             if fill:
