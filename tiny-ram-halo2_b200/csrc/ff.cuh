@@ -8,8 +8,8 @@
 // fuses into IMAD.WIDE.U32(.X).  Products a_j*b_i with even j accumulate in E (limb positions 0..7), odd j
 // in O (positions 1..8); the two are merged once at the end.  Both Pasta moduli have 32-bit limbs
 //     [1, p1, p2, p3, 0, 0, 0, 0x40000000]   and   -p^-1 mod 2^32 = 0xffffffff,
-// so a reduction round is m = -T0, three wide MACs (p1,p2,p3), a carry ripple and one shift pair for the
-// 2^254 term: 88 wide MACs per product instead of 128.
+// so a reduction round is m = -T0, three wide MACs (p1,p2,p3), one carry ripple to the top and one funnel
+// shift for the 2^254 term (see redc_row): 88 wide MACs per product instead of 128.
 //
 // Every asm block below has a plain-C twin (used when compiled for the host) so the carry logic is
 // unit-tested on the CPU build box (tests/test_ff_host.py) before going to the GPU.
@@ -150,58 +150,78 @@ FF_HD void mul_row(uint32_t* En, uint32_t* On, const uint32_t* E, const uint32_t
 }
 
 // One Montgomery reduction round on (E, O): adds m*p with m = -E[0] so that position 0 becomes zero.
-// E[0] is left stale (callers ignore it).
+// E[0] is left stale (callers ignore it).  `mprev` is the previous round's m (0 before round 0) and is
+// replaced by this round's.
+//
+// p = 1 + P1*2^32 + P2*2^64 + P3*2^96 + 2^254, so m*p touches positions 0..4 and 7..8 only.  Positions
+// are 32-bit limbs of the running value; E[k] sits at position k, O[k] at position k+1.
+//   * m*P2 (positions 2,3) goes into E; its carry is taken one limb further (E4, position 4) and caught
+//     in cE.  m*P1 (1,2) and m*P3 (3,4) go into O in one chain that starts from the carry of E0 + m
+//     (E0 + m is 0 or 2^32) and adds cE at position 5.  That O chain is the only ripple to the top; it
+//     passes the zero limbs 5..6 of p once per round instead of once per chain.  (Each product lands on
+//     an even-aligned register pair, E2:E3, O0:O1, O2:O3, which ptxas fuses into one IMAD.WIDE.)
+//   * m*2^254 is m<<30 at position 7 and m>>2 at position 8.  Position 8 of this round is position 7 of
+//     the next, where the next round's m<<30 lands too, so the two share a word:
+//         w = (mprev >> 2) | (m << 30)   (one funnel shift; the bit ranges are disjoint, no carry)
+//     added at position 7 by the same O chain.  Deferring mprev>>2 by one round is safe because position
+//     8 of round i is absolute limb i+8 >= 8: no later m reads it.  The last round's m>>2 is added by
+//     merge_eo.
+// Bounds: with a, b < p every CIOS round keeps the shifted value U < 2p (U' = (U + a*bi + m*p)/2^32 <
+// (2p + 2*(2^32-1)*p)/2^32 < 2p), so before the shift the value is < 2p*2^32 < 2^288 and fits positions
+// 0..8.  The deferred m>>2 only makes the represented value smaller.  Every carry is either consumed in
+// a chain or caught (cE), none is dropped except the last one out of position 8 (O7), which is zero
+// because the value represented by E, O and cE is < 2^288 and every limb is non-negative.
 template <class PR>
-FF_HD void redc_row(uint32_t* E, uint32_t* O) {
+FF_HD void redc_row(uint32_t* E, uint32_t* O, uint32_t& mprev) {
   uint32_t m = 0u - E[0];
-  uint32_t mlo = m << 30, mhi = m >> 2;
 #ifdef __CUDA_ARCH__
-  uint32_t junk;
-  asm("add.cc.u32     %16, %0, %17;\n\t"         // E0 + m -> carry = (E0 != 0)
-      "addc.cc.u32     %1, %1, 0;\n\t"
-      "madc.lo.cc.u32  %2, %17, %21, %2;\n\t"    // m*p2
-      "madc.hi.cc.u32  %3, %17, %21, %3;\n\t"
-      "addc.cc.u32     %4, %4, 0;\n\t"
-      "addc.cc.u32     %5, %5, 0;\n\t"
-      "addc.cc.u32     %6, %6, 0;\n\t"
-      "addc.cc.u32     %7, %7, 0;\n\t"
-      "addc.u32       %15, %15, 0;\n\t"
-      "mad.lo.cc.u32   %8, %17, %20, %8;\n\t"    // m*p1
-      "madc.hi.cc.u32  %9, %17, %20, %9;\n\t"
-      "madc.lo.cc.u32 %10, %17, %22, %10;\n\t"   // m*p3
-      "madc.hi.cc.u32 %11, %17, %22, %11;\n\t"
-      "addc.cc.u32    %12, %12, 0;\n\t"
-      "addc.cc.u32    %13, %13, 0;\n\t"
-      "addc.cc.u32    %14, %14, %18;\n\t"        // + m<<30
-      "addc.u32       %15, %15, %19;"            // + m>>2
-      : "+r"(E[0]), "+r"(E[1]), "+r"(E[2]), "+r"(E[3]), "+r"(E[4]), "+r"(E[5]), "+r"(E[6]), "+r"(E[7]),
-        "+r"(O[0]), "+r"(O[1]), "+r"(O[2]), "+r"(O[3]), "+r"(O[4]), "+r"(O[5]), "+r"(O[6]), "+r"(O[7]),
-        "=&r"(junk)
-      : "r"(m), "r"(mlo), "r"(mhi), "r"(PR::P1), "r"(PR::P2), "r"(PR::P3));
+  uint32_t w = __funnelshift_r(mprev, m, 2);
+  uint32_t cE, junk;
+  asm("mad.lo.cc.u32   %0, %14, %16, %0;\n\t"    // E2 += m*p2 (positions 2, 3)
+      "madc.hi.cc.u32  %1, %14, %16, %1;\n\t"
+      "addc.cc.u32     %2, %2, 0;\n\t"           // E4 (position 4)
+      "addc.u32       %11, 0, 0;\n\t"            // cE: carry into position 5
+      "add.cc.u32     %12, %13, %14;\n\t"        // E0 + m -> carry = (E0 != 0)
+      "madc.lo.cc.u32  %3, %14, %15, %3;\n\t"    // O0 += m*p1 (positions 1, 2)
+      "madc.hi.cc.u32  %4, %14, %15, %4;\n\t"
+      "madc.lo.cc.u32  %5, %14, %17, %5;\n\t"    // O2 += m*p3 (positions 3, 4)
+      "madc.hi.cc.u32  %6, %14, %17, %6;\n\t"
+      "addc.cc.u32     %7, %7, %11;\n\t"         // O4 += cE (position 5)
+      "addc.cc.u32     %8, %8, 0;\n\t"
+      "addc.cc.u32     %9, %9, %18;\n\t"         // O6 += w (position 7)
+      "addc.u32       %10, %10, 0;"              // O7 (position 8)
+      : "+r"(E[2]), "+r"(E[3]), "+r"(E[4]),                                                          // 0..2
+        "+r"(O[0]), "+r"(O[1]), "+r"(O[2]), "+r"(O[3]), "+r"(O[4]), "+r"(O[5]), "+r"(O[6]), "+r"(O[7]),  // 3..10
+        "=&r"(cE), "=&r"(junk)                                                                       // 11, 12
+      : "r"(E[0]), "r"(m), "r"(PR::P1), "r"(PR::P2), "r"(PR::P3), "r"(w));                         // 13..18
 #else
+  uint32_t w = (mprev >> 2) | (m << 30);
   uint64_t t, carry;
-  t = (uint64_t)E[0] + m; carry = t >> 32;
-  t = (uint64_t)E[1] + carry; E[1] = (uint32_t)t; carry = t >> 32;
+  // E: m*p2 at positions 2, 3, one more limb, carry caught in cE
   uint64_t prod = (uint64_t)m * PR::P2;
-  t = (uint64_t)(uint32_t)prod + E[2] + carry; E[2] = (uint32_t)t; carry = t >> 32;
+  t = (uint64_t)(uint32_t)prod + E[2]; E[2] = (uint32_t)t; carry = t >> 32;
   t = (prod >> 32) + E[3] + carry; E[3] = (uint32_t)t; carry = t >> 32;
-  for (int i = 4; i < 8; ++i) { t = (uint64_t)E[i] + carry; E[i] = (uint32_t)t; carry = t >> 32; }
-  O[7] += (uint32_t)carry;
+  t = (uint64_t)E[4] + carry; E[4] = (uint32_t)t; carry = t >> 32;
+  uint32_t cE = (uint32_t)carry;
+  // O: m at position 0, m*p1, m*p3, cE, w, up to position 8
+  t = (uint64_t)E[0] + m; carry = t >> 32;
   prod = (uint64_t)m * PR::P1;
-  t = (uint64_t)(uint32_t)prod + O[0]; O[0] = (uint32_t)t; carry = t >> 32;
+  t = (uint64_t)(uint32_t)prod + O[0] + carry; O[0] = (uint32_t)t; carry = t >> 32;
   t = (prod >> 32) + O[1] + carry; O[1] = (uint32_t)t; carry = t >> 32;
   prod = (uint64_t)m * PR::P3;
   t = (uint64_t)(uint32_t)prod + O[2] + carry; O[2] = (uint32_t)t; carry = t >> 32;
   t = (prod >> 32) + O[3] + carry; O[3] = (uint32_t)t; carry = t >> 32;
-  t = (uint64_t)O[4] + carry; O[4] = (uint32_t)t; carry = t >> 32;
+  t = (uint64_t)O[4] + cE + carry; O[4] = (uint32_t)t; carry = t >> 32;
   t = (uint64_t)O[5] + carry; O[5] = (uint32_t)t; carry = t >> 32;
-  t = (uint64_t)O[6] + mlo + carry; O[6] = (uint32_t)t; carry = t >> 32;
-  O[7] += mhi + (uint32_t)carry;
+  t = (uint64_t)O[6] + w + carry; O[6] = (uint32_t)t; carry = t >> 32;
+  O[7] += (uint32_t)carry;
 #endif
+  mprev = m;
 }
 
-// r = (O + (E >> one limb)), 8 limbs (the value is < 2p < 2^256, so no carry out)
-FF_HD void merge_eo(uint32_t* r, const uint32_t* E, const uint32_t* O) {
+// r = O + (E >> one limb) + top * 2^224, 8 limbs (the value is < 2p < 2^256, so no carry out).  `top` is the
+// last reduction round's m >> 2 (see redc_row).
+FF_HD void merge_eo(uint32_t* r, const uint32_t* E, const uint32_t* O, uint32_t top) {
 #ifdef __CUDA_ARCH__
   asm("add.cc.u32  %0, %8, %16;\n\t"
       "addc.cc.u32 %1, %9, %17;\n\t"
@@ -210,13 +230,13 @@ FF_HD void merge_eo(uint32_t* r, const uint32_t* E, const uint32_t* O) {
       "addc.cc.u32 %4, %12, %20;\n\t"
       "addc.cc.u32 %5, %13, %21;\n\t"
       "addc.cc.u32 %6, %14, %22;\n\t"
-      "addc.u32    %7, %15, 0;"
+      "addc.u32    %7, %15, %23;"
       : "=&r"(r[0]), "=&r"(r[1]), "=&r"(r[2]), "=&r"(r[3]), "=&r"(r[4]), "=&r"(r[5]), "=&r"(r[6]), "=&r"(r[7])
       : "r"(O[0]), "r"(O[1]), "r"(O[2]), "r"(O[3]), "r"(O[4]), "r"(O[5]), "r"(O[6]), "r"(O[7]),
-        "r"(E[1]), "r"(E[2]), "r"(E[3]), "r"(E[4]), "r"(E[5]), "r"(E[6]), "r"(E[7]));
+        "r"(E[1]), "r"(E[2]), "r"(E[3]), "r"(E[4]), "r"(E[5]), "r"(E[6]), "r"(E[7]), "r"(top));
 #else
   uint64_t t = 0;
-  for (int i = 0; i < 8; ++i) { t += (uint64_t)O[i] + (i < 7 ? E[i + 1] : 0); r[i] = (uint32_t)t; t >>= 32; }
+  for (int i = 0; i < 8; ++i) { t += (uint64_t)O[i] + (i < 7 ? E[i + 1] : top); r[i] = (uint32_t)t; t >>= 32; }
 #endif
 }
 
@@ -268,18 +288,19 @@ template <class PR> FF_HD Fe<PR> fe_mul(const Fe<PR>& a, const Fe<PR>& b) {
     E[2 * j] = (uint32_t)pe; E[2 * j + 1] = (uint32_t)(pe >> 32);
     O[2 * j] = (uint32_t)po; O[2 * j + 1] = (uint32_t)(po >> 32);
   }
-  redc_row<PR>(E, O);
+  uint32_t m = 0;
+  redc_row<PR>(E, O, m);
 #pragma unroll
   for (int i = 1; i < 8; i += 2) {
     mul_row(E2, O2, E, O, a.v, b.v[i]);
-    redc_row<PR>(E2, O2);
+    redc_row<PR>(E2, O2, m);
     if (i + 1 < 8) {
       mul_row(E, O, E2, O2, a.v, b.v[i + 1]);
-      redc_row<PR>(E, O);
+      redc_row<PR>(E, O, m);
     }
   }
   Fe<PR> r;
-  merge_eo(r.v, E2, O2);
+  merge_eo(r.v, E2, O2, m >> 2);
   fe_final_sub(r);
   return r;
 }
