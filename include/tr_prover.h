@@ -225,6 +225,35 @@ int trp_dev_permute_expression_pair(trp_ctx* ctx, const uint64_t* d_input, const
 int trp_permute_expression_pair(trp_ctx* ctx, const uint64_t* input, const uint64_t* table, size_t rows, uint64_t* perm_input,
                                 uint64_t* perm_table, int* all_found);
 
+/* ---- witness synthesis (SURVEY.md 8(f) row f4): the TinyRAM circuit's witness block from an execution trace ---------------------
+ * tinyram.TinyRamCircuit.synthesize + program_instance + HostWitness.upload of the Python package (the reference's
+ * ExeChip::assign_trace, tables/exe.rs:792-1080, and ProgConfig, tables/prog.rs:38-60, 195-233), bit for bit.  d_out receives the
+ * (n_cols, n, 4) block of Montgomery columns that create_proof takes: the instance columns, then the advice columns in
+ * constraint-system order, zero outside the assigned rows.  W = word_bits in {8, 16, 24, 32}, R = reg_count, L = 9 R + 22 (the
+ * cells of one program line), TABLE_LEN = 2^(W/2) <= n; n_steps <= TABLE_LEN - 1.  Every value below is a uint64 word.
+ *   steps    n_steps x (4 + R): pc, flag, v_addr (0 where the step has none), instruction index, regs[R] (each < 2^32)
+ *   ins      n_ins x (16 + L + 13), one row per distinct instruction:
+ *              [0] opcode (trace.OPCODES)  [1] ri  [2] rj  (0 where absent)  [3] 1 if operand a is a register  [4] its index, or the
+ *              immediate (< 2^32)  [5..8] the kind of selection a, b, c, d (0 Unset, 1 Zero, 2 Reg, 3 RegN, 4 A, 5 Pc, 6 PcN,
+ *              7 PcPlusOne, 8 VAddr, 9 MaxWord, 10 One, 11 NonDet)  [9..12] the register of a Reg / RegN selection  [13..15] 0;
+ *              then the L values of the program line (ProgramLine::assign_cells, in ProgramLine::to_vec order) and the 13 flags of
+ *              the Out row (Out::new order: and xor or sum prod ssum sprod mod shift flag1 flag2 flag3 flag4)
+ *   prog     prog_len instruction indices, the program in order (rows >= prog_len of the program table repeat the last line)
+ *   colmap   uint32 block column of each role: pc, flag, value, s_trace, a_flag; the (word, even, odd) columns of tv_a, tv_b, tv_c,
+ *            tv_d, r_decompose, a_decompose, logic_b, even_sum, odd_sum; for signed_a, signed_b, signed_c the (word, even, odd) of
+ *            its word, msb, word_sigma and the (word, even, odd) of check_sign; a_shift, a_power, lsb_b, b_flag; regs[R]; the 13 Out
+ *            columns; the L columns of the execution table's line, of the program table and of the instance (0xFFFFFFFF for the
+ *            last two without a program table); the number of intermediate (tracked) columns and their list.
+ *   flags    bit 0: reg_operand_value (synthesize's option), bit 1: with a program table (the instance columns and the program table)
+ * The witness generator's own failures are data errors of the trace, not call errors: the call returns TRP_OK with *err_code
+ * = 0, or the first failure synthesize meets with *err_row its row: 1 unhandled non-deterministic advice, 2 a failed next-register
+ * or sign assertion, 3 a step past the last one, 4 a shift >= 64, 5 a negative check_sign of the signed gadget (d_out is then
+ * undefined).  Synchronises the ctx stream. */
+int trp_dev_tinyram_witness(trp_ctx* ctx, unsigned word_bits, unsigned reg_count, int flags, const uint64_t* steps /* host */,
+                            size_t n_steps, const uint64_t* ins /* host */, size_t n_ins, const uint32_t* prog /* host */, size_t prog_len,
+                            const uint32_t* colmap /* host */, size_t colmap_len, uint64_t* d_out, size_t n_cols, size_t n,
+                            uint64_t* err_row, int* err_code);
+
 /* ---- opening phase (SURVEY.md 8(f) row f2): halo2_proofs 0.2.0 arithmetic.rs {eval_polynomial, compute_inner_product,
  * kate_division, parallel_generator_collapse} and the round body of poly/commitment/prover.rs create_proof (the IPA) ------- */
 /* out[j] = sum_i polys[j * stride + i] * x^i, i < n, for j < m: m evaluations at ONE point (the evaluations at x * omega^rot) */

@@ -35,6 +35,7 @@ EXPORTED_SYMBOLS = [
     "trp_dev_eval_polynomials", "trp_dev_eval_polynomials_at", "trp_dev_linear_combination", "trp_eval_polynomial", "trp_dev_inner_products", "trp_compute_inner_product", "trp_dev_powers",
     "trp_dev_kate_division", "trp_kate_division", "trp_dev_random_field", "trp_dev_fold", "trp_dev_ipa_round_scalars", "trp_dev_ipa_s_double", "trp_dev_generator_collapse", "trp_dev_msm_var",
     "trp_dev_hash_to_curve", "trp_hash_to_curve", "trp_dev_group_fft", "trp_group_fft", "trp_params_new", "trp_dev_params_new",
+    "trp_dev_tinyram_witness",
 ]
 
 
@@ -149,6 +150,8 @@ def load_library():
     L.trp_group_fft.argtypes = [vp, vp, u, vp, vp]
     L.trp_params_new.argtypes = [vp, u, vp, vp, vp, vp]
     L.trp_dev_params_new.argtypes = [vp, u, vp, vp, vp]
+    L.trp_dev_tinyram_witness.argtypes = [vp, u, u, i, vp, sz, vp, sz, vp, sz, vp, sz, vp, sz, sz, ctypes.POINTER(ctypes.c_uint64),
+                                          ctypes.POINTER(i)]
     _lib = L
     return L
 

@@ -192,6 +192,11 @@ def decompose(word: int) -> Tuple[int, int]:
 _NO_GADGET = frozenset(("Add", "Sub", "Mull", "UMulh", "Cmpa", "Cmpae", "CMov", "Jmp", "CJmp", "CnJmp", "LoadW", "StoreW", "Answer", "Not"))
 
 
+# selection kinds of trp_dev_tinyram_witness's instruction table
+_SEL_KIND = {"Unset": 0, "Zero": 1, "Reg": 2, "RegN": 3, "A": 4, "Pc": 5, "PcN": 6, "PcPlusOne": 7, "VAddr": 8, "MaxWord": 9, "One": 10,
+             "NonDet": 11}
+
+
 def _batch_inverse(values: List[int], p: int) -> List[int]:
     """the inverses modulo p of `values` with ONE modular inversion (prefix products); zeros stay zero"""
     prefix, run = [], 1
@@ -209,14 +214,18 @@ def _batch_inverse(values: List[int], p: int) -> List[int]:
     return out
 
 
-def program_instance(prog: List[T.Instruction], word_bits: int, reg_count: int = 8, arrays: bool = False) -> List[List[int]]:
-    """tables/prog.rs:38-60: the 94 instance columns; the program is padded to TABLE_LEN lines with its terminal Answer.
-    arrays: the columns as uint64 numpy arrays (same values)"""
-    table_len = 1 << (word_bits // 2)
+def _check_program(prog: List[T.Instruction], table_len: int):
     if not prog or prog[-1].name != "Answer":
         raise ValueError("Empty programs are invalid / the last instruction must be Answer")
     if len(prog) > table_len:
         raise ValueError("program longer than the program table")
+
+
+def program_instance(prog: List[T.Instruction], word_bits: int, reg_count: int = 8, arrays: bool = False) -> List[List[int]]:
+    """tables/prog.rs:38-60: the 94 instance columns; the program is padded to TABLE_LEN lines with its terminal Answer.
+    arrays: the columns as uint64 numpy arrays (same values)"""
+    table_len = 1 << (word_bits // 2)
+    _check_program(prog, table_len)
     counter = iter(range(1 << 30))
     line = ProgramLine(lambda: next(counter), reg_count)
     n_cols = len(line.to_vec())
@@ -706,6 +715,39 @@ class TinyRamCircuit:
             advice[tc][:TL] = col + [0] * (TL - len(col))
         return advice
 
+    def witness_column_map(self):
+        """trp_dev_tinyram_witness's column map (include/tr_prover.h): the block column (instance columns first, then advice) of
+        every cell role the witness generator writes, taken from the configured columns"""
+        import numpy as np
+        n_inst = self.cs.num_instance
+        adv = lambda cols: [n_inst + c for c in cols]
+        even_bits = lambda e: adv((e.word, e.even, e.odd))
+        m = adv((self.pc, self.flag, self.value, self.s_trace, self.a_flag))
+        for cfg in (self.tv_a, self.tv_b, self.tv_c, self.tv_d, self.r_dec, self.a_decomp, self.logic_b, self.even_sum, self.odd_sum):
+            m += even_bits(cfg)
+        for sg in (self.signed_a, self.signed_b, self.signed_c):
+            m += even_bits(sg.word) + adv((sg.msb, sg.word_sigma)) + even_bits(sg.check_sign)
+        m += adv((self.a_shift, self.a_power, self.lsb_b, self.b_flag)) + adv(self.reg) + adv(self.out[nm] for nm in OUT_NAMES)
+        m += adv(self.line.to_vec())
+        if self.with_prog:
+            m += adv(self.prog_table.to_vec()) + self.prog_input.to_vec()
+        else:
+            m += [0xFFFFFFFF] * (2 * len(self.line.to_vec()))
+        m += [len(self.intermediate)] + adv(self.intermediate)
+        return np.array(m, dtype=np.uint32)
+
+    def witness_instruction_row(self, ins: T.Instruction) -> List[int]:
+        """one row of trp_dev_tinyram_witness's instruction table: the decode words of `ins` (its operands and `selections`), the
+        values of its program line (ProgramLine.row_values) and its Out row (OUT)"""
+        a = ins.a
+        if isinstance(a, T.Imm) and not 0 <= a.value < 1 << 32:
+            raise ValueError(f"{ins.name}: immediate {a.value} is not a 32-bit word")
+        sels = selections(ins)[:4]
+        row = [ins.opcode, ins.ri or 0, ins.rj or 0, int(isinstance(a, T.Reg)), a.index if isinstance(a, T.Reg) else a.value]
+        row += [_SEL_KIND[s[0]] for s in sels] + [s[1] if s[0] in ("Reg", "RegN") else 0 for s in sels] + [0, 0, 0]
+        vals = self.line.row_values(ins)
+        return row + [vals[c] for c in self.line.to_vec()] + [int(nm in OUT[ins.name]) for nm in OUT_NAMES]
+
     # ---- witness helpers -------------------------------------------------------------------------------------------------------------
     def _assign_decompose(self, put, cfg: EvenBits, word: int):
         e, o = decompose(word)
@@ -973,3 +1015,94 @@ class HostWitness:
         r2 = be._dev(be._limbs([be.R]))
         be.ctx.check(be.lib.trp_dev_field_op(be.ctx.handle, 0, 2 | 16, out.data_ptr(), r2.data_ptr(), out.data_ptr(), self.ncols * self.n))
         return out
+
+
+# the witness generator's failures (trp_dev_tinyram_witness's err_code) as the exceptions TinyRamCircuit.synthesize raises
+_WITNESS_ERRORS = {1: (RuntimeError, "Unhandled non-deterministic advice"), 2: (AssertionError, "assertion failed"),
+                   3: (IndexError, "list index out of range"), 4: (OverflowError, "attempt to multiply with overflow"),
+                   5: (AssertionError, "assertion failed: cs >= 0")}
+
+
+def witness_error(code: int, row: int) -> Exception:
+    """the exception of a witness generator failure; .row is the trace row synthesize fails at"""
+    cls, msg = _WITNESS_ERRORS[code]
+    e = cls(f"{msg} (trace row {row})")
+    e.row = row
+    return e
+
+
+def witness_inputs(circ: TinyRamCircuit, trace: T.Trace):
+    """The packed inputs of trp_dev_tinyram_witness (include/tr_prover.h) for `trace`: (steps, instructions, program, column map).
+    One instruction row per distinct instruction (the program's, in order, then any other a step executes)."""
+    import numpy as np
+    R = circ.R
+    by_id, by_value, rows = {}, {}, []
+
+    def kind_of(ins):
+        k = by_id.get(id(ins))
+        if k is None:
+            k = by_value.get(ins)
+            if k is None:
+                k = by_value[ins] = len(rows)
+                rows.append(circ.witness_instruction_row(ins))
+            by_id[id(ins)] = k
+        return k
+
+    prog = np.array([kind_of(ins) for ins in trace.prog], dtype=np.uint32)
+    exe = trace.exe
+    steps = np.zeros((len(exe), 4 + R), dtype=np.uint64)
+    if exe:
+        regs = np.array([st.regs for st in exe], dtype=np.int64)
+        if regs.shape != (len(exe), R) or regs.min() < 0 or regs.max() >= 1 << 32:
+            raise ValueError("register values must be 32-bit words, one per register")
+        steps[:, 0] = [st.pc for st in exe]
+        steps[:, 1] = [st.flag for st in exe]
+        steps[:, 2] = [st.v_addr or 0 for st in exe]
+        steps[:, 3] = [kind_of(st.instruction) for st in exe]
+        steps[:, 4:] = regs
+    ins = np.array(rows, dtype=np.uint64).reshape(len(rows), 16 + len(circ.line.to_vec()) + len(OUT_NAMES))
+    return steps, ins, prog, circ.witness_column_map()
+
+
+def device_witness(be, trace: T.Trace, with_prog: bool = True, reg_operand_value: bool = True, out=None, a_flag_rand=None,
+                   public_input=None):
+    """The witness block of `trace` made on the device: bit for bit HostWitness(be, instances + advice).upload(be) after
+    build(PL, trace, k, with_prog=..., reg_operand_value=...), i.e. the (n_instance + n_advice, n, 4) int64 tensor of Montgomery
+    columns (instance columns first, then advice) whose views create_proof takes.  Only the packed steps and two small tables
+    cross PCIe (trp_dev_tinyram_witness); the failures synthesize / program_instance raise are raised here too, with the same
+    exception types (.row: the trace row of a witness generator failure).  out: a block of that shape to reuse.
+    a_flag_rand and public_input are host-synthesis options (build + HostWitness): asking for one is a ValueError."""
+    import ctypes
+    import numpy as np
+    from . import plonk as PL
+    from ._lib import ptr
+    if a_flag_rand is not None or public_input is not None:
+        raise ValueError("a_flag_rand / public_input: synthesize on the host (build + HostWitness)")
+    circ = TinyRamCircuit(PL, trace.word_bits, trace.reg_count, with_prog=with_prog)
+    if circ.table_len > be.n:
+        raise ValueError("NotEnoughRowsAvailable")
+    if len(trace.exe) > circ.table_len - 1:
+        raise ValueError("trace longer than TABLE_LEN - 1")
+    prog_error = None
+    if with_prog:
+        try:
+            _check_program(trace.prog, circ.table_len)
+        except ValueError as e:                   # raised after the witness generator's own failures, as build() orders them
+            prog_error = e
+    steps, ins, prog, colmap = witness_inputs(circ, trace)
+    flags = int(bool(reg_operand_value)) | (2 if with_prog and prog_error is None else 0)
+    torch = be.torch
+    ncols = circ.cs.num_instance + circ.cs.num_advice
+    if out is None:
+        out = torch.empty((ncols, be.n, 4), dtype=torch.int64, device="cuda")
+    elif tuple(out.shape) != (ncols, be.n, 4) or out.dtype != torch.int64 or not out.is_cuda or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int64 cuda tensor of shape {(ncols, be.n, 4)}")
+    row, code = ctypes.c_uint64(), ctypes.c_int()
+    be.ctx.check(be.lib.trp_dev_tinyram_witness(
+        be.ctx.handle, circ.W, circ.R, flags, ptr(np.ascontiguousarray(steps)), len(steps), ptr(ins), len(ins), ptr(prog), len(prog),
+        ptr(colmap), len(colmap), out.data_ptr(), ncols, be.n, ctypes.byref(row), ctypes.byref(code)))
+    if code.value:
+        raise witness_error(code.value, row.value)
+    if prog_error is not None:
+        raise prog_error
+    return out
