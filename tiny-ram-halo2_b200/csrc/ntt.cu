@@ -239,6 +239,165 @@ __global__ void __launch_bounds__(NTT_THREADS, R >= 3 ? 2 : 3) ntt_pass_reg_kern
   }
 }
 
+// ---- specialised register-blocked pass ---------------------------------------------------------------------------------
+// ntt_pass_reg_kernel<PR, 2> with everything the host knows at launch made a template parameter: the stage count S, the tile
+// width C, first / last pass, the scalings and the gathered source.  The radix-4 groups, their stage offsets and the unit
+// counts are then constants; the per-element bit reversal, swizzle and output position become one per-unit base combined
+// with a compile-time offset per element, and no scaling needs a division:
+//   SCALE_ONE    one scalar (period 1), loaded once per thread;
+//   SCALE_TABLE  a table whose period is at least the index range (the index is its own table index).
+// Any other period runs the generic kernel.
+enum : int { SCALE_NONE = 0, SCALE_ONE = 1, SCALE_TABLE = 2, SCALE_GENERAL = 3 };
+
+constexpr unsigned rev_bits(unsigned x, unsigned n) {
+  unsigned r = 0;
+  for (unsigned b = 0; b < n; ++b) r |= ((x >> b) & 1u) << (n - 1 - b);
+  return r;
+}
+
+template <class F, unsigned... G>
+__device__ __forceinline__ void static_for(F&& f, std::integer_sequence<unsigned, G...>) { (f(std::integral_constant<unsigned, G>()), ...); }
+
+template <class PR, unsigned S, unsigned C, bool FIRST, bool LAST, int PRE, int POST, bool GATHER>
+__global__ void __launch_bounds__(NTT_THREADS, 3) ntt_pass_spec_kernel(NttPass p) {
+  extern __shared__ uint4 smem[];
+  constexpr unsigned NELEM = 1u << (S + C), CMASK = (1u << C) - 1;
+  constexpr unsigned NG = (S + 1) / 2;                          // radix-4 groups, a radix-2 one first when S is odd
+  uint4* plane0 = smem;
+  uint4* plane1 = smem + NELEM;
+  const unsigned L = p.L, lo = FIRST ? 0u : p.lo;
+  const unsigned g = blockIdx.x;
+  const uint4* src = GATHER ? p.src_tab[blockIdx.y] : p.src + 2 * (size_t)blockIdx.y * p.src_stride;
+  uint4* dst = p.dst + 2 * (size_t)blockIdx.y * p.dst_stride;
+  unsigned low_base = 0, hi = 0;
+  if (!FIRST) { low_base = (g & ((1u << (lo - C)) - 1)) << C; hi = g >> (lo - C); }
+  Fe<PR> pre_one, post_one;
+  if constexpr (FIRST && PRE == SCALE_ONE) pre_one = fe_load_ro<PR>(p.pre);
+  if constexpr (LAST && POST == SCALE_ONE) post_one = fe_load_ro<PR>(p.post);
+  // the swizzle is XOR-linear in the index: slot(t, i_base | e << q0) = slot(t, i_base) ^ swz(e << q0)
+  auto slot = [&](unsigned t, unsigned i) -> unsigned {
+    const unsigned idx = (t << S) | i;
+    return idx ^ (((idx >> 3) ^ (t << (3 - C))) & 7u);
+  };
+  static_for([&](auto gtag) {
+    constexpr unsigned GI = decltype(gtag)::value;
+    constexpr unsigned RR = (S & 1) && GI == 0 ? 1 : 2;
+    constexpr unsigned Q0 = GI == 0 ? 0 : 2 * GI - (S & 1);
+    constexpr unsigned E = 1u << RR;
+    constexpr bool GFIRST = GI == 0, GLAST = GI + 1 == NG;
+    constexpr unsigned UNITS = NELEM >> RR, TILE_UNITS_LOG = S - RR;
+#pragma unroll 1
+    for (unsigned u = threadIdx.x; u < UNITS; u += NTT_THREADS) {
+      unsigned t, j;
+      if (GLAST && FIRST) { j = u & ((1u << TILE_UNITS_LOG) - 1); t = u >> TILE_UNITS_LOG; }   // contiguous stores along i
+      else { t = u & CMASK; j = u >> C; }                                                        // adjacent tiles adjacent in memory
+      if (GFIRST && FIRST && C) t = __brev(t) >> (32 - C);
+      const unsigned j_low = j & ((1u << Q0) - 1), j_high = j >> Q0;
+      const unsigned i_base = (j_high << (Q0 + RR)) | j_low;
+      Fe<PR> x[E];
+      if constexpr (GFIRST) {
+        // source index of element e: the bit reversal (first pass) maps index bit Q0 + k to bit L - 1 - Q0 - k
+        unsigned sbase, sshift;
+        if constexpr (FIRST) {
+          sbase = L ? __brev((t << (L - C)) | (g << S) | i_base) >> (32 - L) : 0u;
+          sshift = L - Q0 - RR;
+        } else {
+          sbase = (hi << (lo + S)) | (i_base << lo) | low_base | t;
+          sshift = lo + Q0;
+        }
+#pragma unroll
+        for (unsigned e = 0; e < E; ++e) {
+          const unsigned sidx = sbase | ((FIRST ? rev_bits(e, RR) : e) << sshift);
+          if (sidx < p.n_src) {
+            x[e] = fe_load<PR>(src + 2 * (size_t)sidx);
+            if constexpr (PRE == SCALE_ONE) x[e] = fe_mul(x[e], pre_one);
+            else if constexpr (PRE == SCALE_TABLE) x[e] = fe_mul(x[e], fe_load_ro<PR>(p.pre + 2 * (size_t)sidx));
+          } else {
+            x[e] = fe_zero<PR>();
+          }
+        }
+      } else {
+        const unsigned sl = slot(t, i_base);
+#pragma unroll
+        for (unsigned e = 0; e < E; ++e) {
+          const unsigned d = e << Q0;
+          x[e] = lds_fe<PR>(plane0, plane1, sl ^ (d ^ ((d >> 3) & 7u)));
+        }
+      }
+      const unsigned low = FIRST ? 0u : (low_base | t);
+#pragma unroll
+      for (unsigned a = 0; a < RR; ++a) {
+        const unsigned tt = lo + Q0 + a;
+#pragma unroll
+        for (unsigned b = 0; b < E / 2; ++b) {
+          const unsigned el = b & ((1u << a) - 1);
+          const unsigned e0 = ((b >> a) << (a + 1)) | el, e1 = e0 | (1u << a);
+          Fe<PR> y = x[e1];
+          // first group of the first pass: the butterflies with el == 0 multiply by omega^0 = 1 (skipped, bit-identical)
+          if (!(FIRST && GFIRST && el == 0) && tt > 0) {
+            const unsigned expo = (((j_low | (el << Q0)) << lo) | low) << (L - tt - 1);
+            y = fe_mul(y, fe_load_ro<PR>(p.tw + 2 * (size_t)expo));
+          }
+          x[e1] = fe_sub(x[e0], y);
+          x[e0] = fe_add(x[e0], y);
+        }
+      }
+      if constexpr (GLAST) {
+        const unsigned pbase = FIRST ? ((t << (L - C)) | (g << S) | i_base) : ((hi << (lo + S)) | (i_base << lo) | low_base | t);
+        const unsigned pshift = FIRST ? Q0 : lo + Q0;
+#pragma unroll
+        for (unsigned e = 0; e < E; ++e) {
+          const unsigned pos = pbase | (e << pshift);
+          if (LAST && pos >= p.n_dst) continue;
+          Fe<PR> v = x[e];
+          if constexpr (LAST && POST == SCALE_ONE) v = fe_mul(v, post_one);
+          else if constexpr (LAST && POST == SCALE_TABLE) v = fe_mul(v, fe_load_ro<PR>(p.post + 2 * (size_t)pos));
+          fe_store(dst + 2 * (size_t)pos, v);
+        }
+      } else {
+        const unsigned sl = slot(t, i_base);
+#pragma unroll
+        for (unsigned e = 0; e < E; ++e) {
+          const unsigned d = e << Q0;
+          sts_fe(plane0, plane1, sl ^ (d ^ ((d >> 3) & 7u)), x[e]);
+        }
+      }
+    }
+    if constexpr (!GLAST) __syncthreads();
+  }, std::make_integer_sequence<unsigned, NG>());
+}
+
+using PassKernel = void (*)(NttPass);
+
+// The specialised instance for a pass of a two-pass plan, or NULL (middle passes, single-pass transforms, general periods).
+template <class PR, unsigned S, unsigned C>
+PassKernel spec_pass_kernel(const NttPass& p, int pre, int post) {
+  if (p.s != S || p.c != C || p.first == p.last) return nullptr;
+  if (p.first) {
+    if (p.src_tab) {
+      if (pre == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_NONE, SCALE_NONE, true>;
+      if (pre == SCALE_ONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_ONE, SCALE_NONE, true>;
+      if (pre == SCALE_TABLE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_TABLE, SCALE_NONE, true>;
+    } else {
+      if (pre == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_NONE, SCALE_NONE, false>;
+      if (pre == SCALE_ONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_ONE, SCALE_NONE, false>;
+      if (pre == SCALE_TABLE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_TABLE, SCALE_NONE, false>;
+    }
+    return nullptr;
+  }
+  if (post == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_NONE, false>;
+  if (post == SCALE_ONE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_ONE, false>;
+  if (post == SCALE_TABLE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_TABLE, false>;
+  return nullptr;
+}
+
+// how a scaling with this table and period reaches indices below `range`
+int scale_kind(const void* tab, unsigned period, unsigned range) {
+  if (!tab) return SCALE_NONE;
+  if (period <= 1) return SCALE_ONE;
+  return period >= range ? SCALE_TABLE : SCALE_GENERAL;
+}
+
 // ---- TMA-staged pass (sm_100a: cp.async.bulk.tensor + mbarrier) ------------------------------------------------------------------
 // Same pass geometry and the same register-blocked butterflies as ntt_pass_reg_kernel, but the tile reaches shared memory
 // through the TMA unit instead of through registers: the 2^(s+c) elements of a tile are 2^s runs of 2^c adjacent elements
@@ -500,14 +659,30 @@ int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned
     size_t out_stride = p.last ? dst_stride : mid_stride;
     p.src = (const uint4*)in; p.dst = (uint4*)out; p.src_stride = in_stride; p.dst_stride = out_stride;
     p.src_tab = p.first ? (const uint4* const*)d_src_tab : nullptr;
+    // register-blocked kernel, radix-4 groups by default (measured on B200 at 8 x 2^20: radix 4 1.53 ms, radix 8 1.61 ms --
+    // 117 registers cost a CTA per SM --, one stage per barrier 1.58 ms); TRP_NTT_RADIX=8 / 2 select the other two
+    static const int radix_log = [] { const char* e = getenv("TRP_NTT_RADIX"); int v = e ? atoi(e) : 4; return v == 2 ? 1 : v == 8 ? 3 : 2; }();
+    // TMA-staged tile loads (TRP_NTT_TMA=1; profiles/ncu_ntt_r02.md has the A/B)
+    static const bool use_tma = [] { const char* e = getenv("TRP_NTT_TMA"); return e && atoi(e) == 1; }();
+    if (radix_log == 2 && !use_tma) {
+      // the shapes a proof runs (both passes of a size-2^19..2^20 transform) have a specialised instance
+      const int pre_kind = p.first ? scale_kind(p.pre, p.pre_period, p.n_src < N ? p.n_src : (unsigned)N) : SCALE_NONE;
+      const int post_kind = p.last ? scale_kind(p.post, p.post_period, p.n_dst < N ? p.n_dst : (unsigned)N) : SCALE_NONE;
+      if (PassKernel k = spec_pass_kernel<PR, 10, 1>(p, pre_kind, post_kind)) {
+        const size_t sm = (size_t)32 << (p.s + p.c);
+        ProfScope ps(ctx, PROF_NTT_PASS, (double)batch * (double)(N >> 1) * (double)p.s);
+        if (sm > 48 * 1024) TRP_CUDA(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+        k<<<dim3((unsigned)(N >> (p.s + p.c)), (unsigned)batch), NTT_THREADS, sm, ctx->stream>>>(p);
+        TRP_LAUNCHED(ctx);
+        continue;
+      }
+    }
     unsigned nelem = 1u << (p.s + p.c);
     unsigned threads = nelem / 2 < NTT_THREADS ? nelem / 2 : NTT_THREADS;
     if (threads < 32) threads = 32;
     dim3 grid((unsigned)(N >> (p.s + p.c)), (unsigned)batch);
     size_t smem = (size_t)nelem * 32;
-    // register-blocked kernel, radix-4 groups by default (measured on B200 at 8 x 2^20: radix 4 1.53 ms, radix 8 1.61 ms --
-    // 117 registers cost a CTA per SM --, one stage per barrier 1.58 ms); TRP_NTT_RADIX=8 / 2 select the other two
-    static const int radix_log = [] { const char* e = getenv("TRP_NTT_RADIX"); int v = e ? atoi(e) : 4; return v == 2 ? 1 : v == 8 ? 3 : 2; }();
+    // generic register-blocked kernel for every other shape
     ProfScope ps(ctx, PROF_NTT_PASS, (double)batch * (double)(N >> 1) * (double)p.s);      // work = radix-2 butterflies of this pass
     if (p.s == 0 || radix_log == 1) {
       if (smem > 48 * 1024)
@@ -518,7 +693,6 @@ int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned
       if (th < 32) th = 32;
       // TMA-staged tile loads (TRP_NTT_TMA=1; profiles/ncu_ntt_r02.md has the A/B): needs whole rows, so a zero-padded first
       // pass qualifies only when the padding starts on a row boundary
-      static const bool use_tma = [] { const char* e = getenv("TRP_NTT_TMA"); return e && atoi(e) == 1; }();
       const size_t row_len = p.first ? (N >> p.s) : ((size_t)1 << p.lo);
       const size_t rows = p.first ? (p.n_src / row_len) : (N >> p.lo);
       if (use_tma && !p.src_tab && p.s >= 2 && (!p.first || (p.n_src % row_len == 0 && rows >= 1)) && ((uintptr_t)in % 16 == 0)) {
