@@ -42,6 +42,7 @@ g = torch.Generator(device="cuda"); g.manual_seed(7)
 def rnd(b):  # below 2^248: canonical in both Pasta fields
     a = torch.randint(0, 1 << 62, (b, 1 << K, 4), dtype=torch.int64, device="cuda", generator=g)
     a[..., 3] &= (1 << 56) - 1
+    torch.cuda.synchronize()  # written on torch's stream, read on the ctx's: the values must be there before the transform runs
     return a
 a = rnd(8)
 out["fwd8_ms"] = timed(stream, lambda: ctx.check(lib.trp_dev_ntt(ctx.handle, a.data_ptr(), 8, K, ptr(dom.omega))))

@@ -6,7 +6,8 @@ representative best_multiexp returns is not unique on the CPU either)."""
 import numpy as np
 import pytest
 
-from util import O, pm, make_points, scalars_uniform, scalars_tinyram, affine_of, generator
+from util import O, pm, FIELDS, make_points, scalars_uniform, scalars_tinyram, affine_of, generator
+from test_ff_carry_cpu import _edges
 
 pytestmark = pytest.mark.gpu
 
@@ -26,27 +27,31 @@ def ctxs(pkg):
 @pytest.mark.parametrize("curve", [O.VESTA, O.PALLAS])
 @pytest.mark.parametrize("which", [0, 1])
 def test_field_ops(ctxs, curve, which):
+    """every pair of the carry-bound operands of test_ff_carry_cpu (0, 1, p - 1, 2^254 - 1, R, all-ones low limbs, the top word
+    at its maximum, ...) through the device's add, sub and mul, sqr and inv on each of them, then uniform random operands"""
     ctx = ctxs[curve]
     field = O.SCALAR_FIELD[curve] if which == 0 else O.BASE_FIELD[curve]
-    p = O.MODULUS[field]
-    edge = [0, 1, 2, p - 1, p - 2, (1 << 254) - 1, 1 << 254, (1 << 32) - 1, 1 << 32, p >> 1]
-    a = np.concatenate([O.ints_to_limbs(edge), O.random_field_mont(field, 4000, 1)])
-    b = np.concatenate([O.ints_to_limbs(list(reversed(edge))), O.random_field_mont(field, 4000, 2)])
+    edge = _edges(FIELDS[field])
+    a = np.concatenate([O.ints_to_limbs([x for x in edge for _ in edge]), O.random_field_mont(field, 4000, 1)])
+    b = np.concatenate([O.ints_to_limbs([y for _ in edge for y in edge]), O.random_field_mont(field, 4000, 2)])
     for op in ("add", "sub", "mul"):
         assert np.array_equal(ctx.field_op(op, a, b, which_field=which), O.field_op(field, op, a, b)), op
-    assert np.array_equal(ctx.field_op("sqr", a, which_field=which), O.field_op(field, "sqr", a))
-    assert np.array_equal(ctx.field_op("inv", a[:300], which_field=which), O.field_op(field, "inv", a[:300]))
+    one = np.concatenate([O.ints_to_limbs(edge), O.random_field_mont(field, 4000, 3)])
+    assert np.array_equal(ctx.field_op("sqr", one, which_field=which), O.field_op(field, "sqr", one))
+    assert np.array_equal(ctx.field_op("inv", one[:300], which_field=which), O.field_op(field, "inv", one[:300]))
 
 
 # ---- K4 NTT ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("curve", [O.VESTA, O.PALLAS])
-@pytest.mark.parametrize("log_n", [0, 1, 2, 3, 5, 9, 10, 11, 12, 13, 16, 18])
+@pytest.mark.parametrize("log_n", list(range(22)) + [23])
 def test_best_fft(pkg, ctxs, curve, log_n):
+    """every pass plan up to 2^21 and 2^23 (2^22 and 2^24 are below): one pass up to 2^10, two generic passes 2^11 .. 2^18, the
+    specialised first pass with a generic second one at 2^19, both passes specialised at 2^20, three passes from 2^21 on"""
     ctx = ctxs[curve]
     field = O.SCALAR_FIELD[curve]
-    F = {O.FP: pm.Fp, O.FQ: pm.Fq}[field]
+    F = FIELDS[field]
     omega = O.to_mont(field, O.ints_to_limbs([F.root_of_unity(log_n)]))[0]
-    batch = 3 if log_n <= 13 else 1
+    batch = 3 if log_n <= 13 else 2 if log_n <= 20 else 1
     a = O.random_field_mont(field, batch << log_n, 30 + log_n).reshape(batch, 1 << log_n, 4)
     got = pkg.best_fft(ctx, a, omega, log_n)
     for b in range(batch):
@@ -313,19 +318,21 @@ def test_best_multiexp_2_22_2_24(pkg, ctxs, log_n, flags):
         bases.free()
 
 
+@pytest.mark.parametrize("curve", [O.VESTA, O.PALLAS])
 @pytest.mark.parametrize("log_n", [22, 24])
-def test_best_fft_2_22_2_24(pkg, ctxs, log_n):
-    ctx = ctxs[O.VESTA]
-    omega = O.to_mont(O.FP, O.ints_to_limbs([pm.Fp.root_of_unity(log_n)]))[0]
-    a = O.random_field_mont(O.FP, 1 << log_n, 30 + log_n)
+def test_best_fft_2_22_2_24(pkg, ctxs, curve, log_n):
+    ctx = ctxs[curve]
+    field = O.SCALAR_FIELD[curve]
+    omega = O.to_mont(field, O.ints_to_limbs([FIELDS[field].root_of_unity(log_n)]))[0]
+    a = O.random_field_mont(field, 1 << log_n, 30 + log_n)
     got = pkg.best_fft(ctx, a, omega, log_n)
-    want = O.fft(O.FP, a, log_n, omega)
+    want = O.fft(field, a, log_n, omega)
     assert np.array_equal(got, want)
     # and back: the inverse transform with omega^-1, scaled by 2^-log_n, returns the input (size-independent property)
-    omega_inv = O.field_op(O.FP, "inv", omega.reshape(1, 4))[0]
+    omega_inv = O.field_op(field, "inv", omega.reshape(1, 4))[0]
     back = pkg.best_fft(ctx, got, omega_inv, log_n)
-    ninv = O.to_mont(O.FP, O.ints_to_limbs([pow(1 << log_n, -1, O.MODULUS[O.FP])]))
-    assert np.array_equal(O.field_op(O.FP, "mul", back, np.repeat(ninv, 1 << log_n, axis=0)), a)
+    ninv = O.to_mont(field, O.ints_to_limbs([pow(1 << log_n, -1, O.MODULUS[field])]))
+    assert np.array_equal(O.field_op(field, "mul", back, np.repeat(ninv, 1 << log_n, axis=0)), a)
 
 
 @pytest.mark.parametrize("k", [20, 22])

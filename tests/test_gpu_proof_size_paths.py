@@ -1,9 +1,11 @@
 """GPU tests of the paths a proof takes only at proof size, each against the oracle:
 
 - trp_dev_coeff_to_coset_gather (the quotient's coset NTTs reading their columns through a device table of addresses): scattered,
-  repeated and interior-row sources, every coset index, single- and multi-pass sizes, k = 20, and the 65 535-column chunking;
+  repeated and interior-row sources, every coset index, single- and multi-pass sizes, k = 19 and 20 in both fields (with
+  trp_dev_coeff_to_coset in and out of place), and the 65 535-column chunking;
 - trp_dev_cosets_to_coeff_parts (a quotient given as a sum of parts of different degrees): the prover's part shape and others,
-  more than 8 output pieces (a second row of the combine grid), the most parts the entry point takes;
+  more than 8 output pieces (a second row of the combine grid), the most parts the entry point takes, the prover's shape at
+  k = 19 and 20;
 - GpuBackend._commit_many at k = 18, where the backend keeps a narrow c = 13 table over g_lagrange ++ [w] for mostly-zero columns
   and commits grand-product columns by parts over the prefix sums of g_lagrange: which table each batch takes, and every
   commitment against the oracle's MSM over g_lagrange ++ [w];
@@ -85,14 +87,26 @@ def test_coset_gather_against_the_oracle(pkg, ctxs, curve, j, k):
 
 
 def test_coset_gather_k20(pkg, ctxs):
-    """two columns at k = 20 (the quotient's size in the benchmark) on the first and the last coset, against the oracle and
-    against trp_dev_coeff_to_coset on a contiguous copy"""
+    """Vesta at k = 20, the quotient's size in the benchmark (_coset_gather_at_proof_size)"""
+    _coset_gather_at_proof_size(pkg, ctxs, O.VESTA, 20)
+
+
+@pytest.mark.parametrize("curve,k", [(O.PALLAS, 20), (O.VESTA, 19), (O.PALLAS, 19)])
+def test_coset_gather_k19_k20(pkg, ctxs, curve, k):
+    """the other field, and k = 19, where only the first pass is specialised (_coset_gather_at_proof_size)"""
+    _coset_gather_at_proof_size(pkg, ctxs, curve, k)
+
+
+def _coset_gather_at_proof_size(pkg, ctxs, curve, k):
+    """two columns (the specialised first pass reads them through the table at k = 19 and 20) on the first and the last coset,
+    against the oracle, and trp_dev_coeff_to_coset on a contiguous copy against the oracle too: out of place (the destination
+    holds the intermediate) and in place (through the scratch buffer)"""
     import torch
-    ctx, field, j, k = ctxs[O.VESTA], O.FP, 6, 20
+    ctx, field, j = ctxs[curve], O.SCALAR_FIELD[curve], 6
     dom = pkg.EvaluationDomain(ctx, j, k)
     n = 1 << k
     period = dom.extended_len() // n
-    host = O.random_field_mont(field, 2 * n, 320).reshape(2, n, 4)
+    host = O.random_field_mont(field, 2 * n, 320 + k).reshape(2, n, 4)
     ext = O.coeff_to_extended(field, j, k, host)
     big = _dev(np.concatenate([host[0], O.random_field_mont(field, 5, 3)]))     # column 0 at row 0 of a longer tensor
     own = _dev(host[1])
@@ -100,15 +114,22 @@ def test_coset_gather_k20(pkg, ctxs):
     out = torch.empty((2, n, 4), dtype=torch.int64, device="cuda")
     ref = torch.empty_like(out)
     for cs in (0, period - 1):
+        want = np.stack([ext[1, cs::period], ext[0, cs::period]])
         out.fill_(-1)
         assert _gather(ctx, dom, [own.data_ptr(), big.data_ptr()], out, cs) == 0
-        got = _u64(out)
-        assert np.array_equal(got, ext[[1, 0]][:, cs::period]), cs
+        assert np.array_equal(_u64(out), want), cs
+        ref.fill_(-1)
         torch.cuda.synchronize()
         ctx.check(ctx.lib.trp_dev_coeff_to_coset(dom.handle, contiguous.data_ptr(), ref.data_ptr(), 2, cs))
         ctx.sync()
-        assert np.array_equal(_u64(ref), got), cs
+        assert np.array_equal(_u64(ref), want), cs
+        ref.copy_(contiguous)
+        torch.cuda.synchronize()
+        ctx.check(ctx.lib.trp_dev_coeff_to_coset(dom.handle, ref.data_ptr(), ref.data_ptr(), 2, cs))
+        ctx.sync()
+        assert np.array_equal(_u64(ref), want), ("in place", cs)
     assert np.array_equal(_u64(own), host[1]) and np.array_equal(_u64(big[:n]), host[0])
+    assert np.array_equal(_u64(contiguous), host[[1, 0]])
     dom.free()
     del ext, out, ref, big, own, contiguous
     torch.cuda.empty_cache()
@@ -187,10 +208,19 @@ PART_SHAPES = [(6, [1, 2, 3, 4, 5], 5),           # the prover's shape (degrees 
                (17, [1, 16, 3, 9], 16)]           # parts below that row come first: its threads must still step over them
 
 
-@pytest.mark.parametrize("curve", [O.VESTA, O.PALLAS])
-@pytest.mark.parametrize("k", [3, 10, 11, 14])
-@pytest.mark.parametrize("divide", [0, 1])
-@pytest.mark.parametrize("shape", range(len(PART_SHAPES)), ids=lambda i: "j%d-%s-out%d" % (PART_SHAPES[i][0], "_".join(map(str, PART_SHAPES[i][1])), PART_SHAPES[i][2]))
+def _parts_case(curve, k, divide, shape, **kw):
+    j, parts, ncos_out = PART_SHAPES[shape]
+    return pytest.param(curve, k, divide, shape, id="j%d-%s-out%d-%d-%d-%d" % (j, "_".join(map(str, parts)), ncos_out, divide, k, curve), **kw)
+
+
+# every shape at k = 3 .. 14, and the prover's shape at k = 19 and 20 (the specialised pass: at k = 20 the last one scales by the
+# table of coset-power inverses) with the division, and at k = 19 without it
+PARTS_CASES = [_parts_case(curve, k, divide, shape) for shape in range(len(PART_SHAPES)) for divide in (0, 1) for k in (3, 10, 11, 14)
+               for curve in (O.VESTA, O.PALLAS)]
+PARTS_CASES += [_parts_case(curve, k, divide, 0) for k, divide in ((19, 1), (20, 1), (19, 0)) for curve in (O.VESTA, O.PALLAS)]
+
+
+@pytest.mark.parametrize("curve,k,divide,shape", PARTS_CASES)
 def test_cosets_to_coeff_parts_against_the_oracle(pkg, ctxs, curve, k, divide, shape):
     """part p: random coefficients a_p of degree < Q_p n, its values on cosets 0 .. Q_p - 1 (times gamma_i - 1 with the vanishing
     division); the result must be sum_p a_p, zero-padded to ncos_out pieces.  k = 11 and 14 take the multi-pass inverse NTT."""
@@ -225,6 +255,9 @@ def test_cosets_to_coeff_parts_against_the_oracle(pkg, ctxs, curve, k, divide, s
         ctx.sync()
         assert np.array_equal(_u64(one), got[:Q * n])
     dom.free()
+    if k >= 19:
+        del d_vals, out
+        torch.cuda.empty_cache()
 
 
 @pytest.mark.parametrize("k", [3, 11])

@@ -369,14 +369,16 @@ __global__ void __launch_bounds__(NTT_THREADS, 3) ntt_pass_spec_kernel(NttPass p
 
 using PassKernel = void (*)(NttPass);
 
-// The specialised instance for a pass of a two-pass plan, or NULL (middle passes, single-pass transforms, general periods).
+// The specialised instance for a pass of a two-pass plan, or NULL (middle passes, single-pass transforms, general periods,
+// a zero-padded first pass or a truncated last pass: coeff_to_extended pads and extended_to_coeff truncates, both with a
+// period-3 scaling that the generic kernel runs anyway).  A gathered source is always scaled by a table of n coset powers.
 template <class PR, unsigned S, unsigned C>
 PassKernel spec_pass_kernel(const NttPass& p, int pre, int post) {
   if (p.s != S || p.c != C || p.first == p.last) return nullptr;
+  const unsigned N = 1u << p.L;
   if (p.first) {
+    if (p.n_src < N) return nullptr;
     if (p.src_tab) {
-      if (pre == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_NONE, SCALE_NONE, true>;
-      if (pre == SCALE_ONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_ONE, SCALE_NONE, true>;
       if (pre == SCALE_TABLE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_TABLE, SCALE_NONE, true>;
     } else {
       if (pre == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, true, false, SCALE_NONE, SCALE_NONE, false>;
@@ -385,6 +387,7 @@ PassKernel spec_pass_kernel(const NttPass& p, int pre, int post) {
     }
     return nullptr;
   }
+  if (p.n_dst < N) return nullptr;
   if (post == SCALE_NONE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_NONE, false>;
   if (post == SCALE_ONE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_ONE, false>;
   if (post == SCALE_TABLE) return ntt_pass_spec_kernel<PR, S, C, false, true, SCALE_NONE, SCALE_TABLE, false>;
@@ -665,7 +668,8 @@ int ntt_run(trp_ctx* ctx, const void* d_src, void* d_dst, size_t batch, unsigned
     // TMA-staged tile loads (TRP_NTT_TMA=1; profiles/ncu_ntt_r02.md has the A/B)
     static const bool use_tma = [] { const char* e = getenv("TRP_NTT_TMA"); return e && atoi(e) == 1; }();
     if (radix_log == 2 && !use_tma) {
-      // the shapes a proof runs (both passes of a size-2^19..2^20 transform) have a specialised instance
+      // the shapes a proof runs have a specialised instance: both passes of a size-2^20 transform, the first pass of a
+      // size-2^19 one (its second pass, s = 9 and c = 2, runs the generic kernel)
       const int pre_kind = p.first ? scale_kind(p.pre, p.pre_period, p.n_src < N ? p.n_src : (unsigned)N) : SCALE_NONE;
       const int post_kind = p.last ? scale_kind(p.post, p.post_period, p.n_dst < N ? p.n_dst : (unsigned)N) : SCALE_NONE;
       if (PassKernel k = spec_pass_kernel<PR, 10, 1>(p, pre_kind, post_kind)) {
